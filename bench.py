@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W           (N > 1: launched by torchrun)
     python bench.py --impl reference ...                    (CPU arm: the oracle port on the host cores)
+    python bench.py ... --dump-outputs DIR                  (+ the last timed step's outputs as DIR/<name>.npy)
 
 Prints ONE JSON line (rank 0).  Workload = BASELINE.json configs[2]: 4096 rays per GPU
 drawn from the 800x800 config-2 camera, two view-direction D=8/W=256 MLPs, L=10/4
@@ -109,6 +110,19 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_step_outputs(out_dir, tr):
+    """What the last training step computed, as float32 DIR/<name>.npy (about 10 MB in all): its loss, the fine and
+    coarse colours of the ray batch, the all-reduced gradient bucket and the parameters after its Adam update (the
+    last two: coarse then fine network, named_parameters() order, flattened).  The rays, targets, initial weights and
+    jitter seed are fixed, so two builds run with the same arguments can be compared array for array."""
+    import numpy as np
+    pl = tr._plans[RAYS_PER_GPU]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in (("loss", tr._loss), ("rgb_map", pl.rgb), ("rgb0", pl.rgb0), ("grads", tr.bucket.grad),
+                    ("params", tr.bucket.flat)):
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
 
 
 def cpu_step_sample(n_rays, threads, steps, warmup):
@@ -296,7 +310,12 @@ def main():
                          "merge -> raw2outputs(192) on 4096 rays, GPU chain beside the CPU oracle (parity-test sized)")
     ap.add_argument("--cfg2", action="store_true", help="BASELINE configs[1]: 800x800 inference render, rows sharded over the ranks")
     ap.add_argument("--cfg4", action="store_true", help="BASELINE configs[3]: 8 views 1024^2 x 192 samples, views sharded over the ranks")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="training step only: after the timed steps, rank 0 writes what the last of them computed as "
+                         "DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl == "reference" or args.cfg1 or args.cfg2 or args.cfg4):
+        ap.error("--dump-outputs applies to the training-step benchmark only")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -325,6 +344,10 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
     warm = max(args.warmup, 3)
     K, c2w = orbit_camera()
+    # NerfTrainer draws the Philox seed of the jitter and importance uniforms from torch's global generator, whose
+    # start-up seed differs from process to process (torch 2.11): seed it (0 + rank, like the ray selection) so
+    # that every run draws the same samples
+    torch.manual_seed(rank)
     tr = NerfTrainer(800, 800, K, c2w, near=2.0, far=6.0, N_samples=N_SAMPLES, N_importance=N_IMPORTANCE,
                      perturb=1.0, white_bkgd=True, device=dev, seed=0)
     # per-rank synthetic batches (seed 0 + rank), resident on the device and mirrored in pinned host memory
@@ -381,6 +404,8 @@ def main():
 
     # ---- device-resident inputs ("value"): the captured step, no per-kernel timers ----
     ms, clocks, launches, _ = timed(lambda i: tr.step(idx_d[i % NB], tgt_d[i % NB]), args.steps, False)
+    if args.dump_outputs and rank == 0:       # before the passes below train the networks further
+        dump_step_outputs(args.dump_outputs, tr)
     value = RAYS_PER_GPU * world * args.steps / (ms * 1e-3)
     # ---- end to end through the public API with host buffers ----
     # Every step copies its ray ids + targets from pinned host memory and its loss is read on the host; the host

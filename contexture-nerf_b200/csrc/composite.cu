@@ -196,7 +196,7 @@ composite_fwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
 // also yields rgb_map, so the photometric loss img2mse(rgb_map, target) (src/run_nerf_helpers.py:9) and its
 // gradient g_rgb = 2 (rgb_map - target) * loss_scale are formed in place -- one pass over raw replaces
 // composite_fwd + mse + composite_bwd.  It writes g_raw, optionally weights (the coarse pass feeds sample_pdf) and
-// rgb_map, and adds sum((rgb-target)^2) * loss_scale into loss[0] (one atomic per warp pass).
+// rgb_map; the loss itself is summed from rgb_map by loss_sum_kernel, in a fixed order.
 template <int K, int G, bool TRAIN>
 __global__ void __launch_bounds__(kCompWarps * 32, K <= 4 ? 4 : (K <= 8 ? 2 : 1))
 composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z,
@@ -212,7 +212,6 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
   const int64_t warp0 = (int64_t)blockIdx.x * kCompWarps + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * kCompWarps;
   const int s0 = lane * K;
-  float loss_acc = 0.f;                              // TRAIN: this lane's share of the loss over all its rays
   for (int64_t rb = warp0 * RPW; rb < R; rb += nwarps * RPW) {
     const bool live = rb + sub < R;
     const int64_t ray = live ? rb + sub : R - 1;
@@ -283,8 +282,6 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
       if (lane == 0 && live) {
         if (rgb_out != nullptr) { rgb_out[ray * 3 + 0] = sr + bg; rgb_out[ray * 3 + 1] = sg + bg; rgb_out[ray * 3 + 2] = sb + bg; }
       }
-      // loss: one value per ray (lane 0 of each live group), kept in a register over the grid-stride loop
-      if (lane == 0 && live) loss_acc += (er * er + eg * eg + eb * eb) * loss_scale;
     } else {
 #pragma unroll
       for (int k = 0; k < K; ++k) {
@@ -359,10 +356,6 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
         U = Gs[k] * alpha + ((1.0f - alpha) + 1e-10f) * U;
       }
     }
-  }
-  if constexpr (TRAIN) {                             // one atomic per warp for the whole launch
-    loss_acc = warp_sum(loss_acc);
-    if ((threadIdx.x & 31) == 0 && loss_acc != 0.f) atomicAdd(loss, loss_acc);
   }
 }
 
@@ -476,7 +469,6 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
   const int64_t nwarps = (int64_t)gridDim.x * kCompWarps;
   const int n_chunks = (S + 32 * K - 1) / (32 * K);
   const int vec = dev_vec(S, z, noise, TRAIN ? (const void*)weights_out : (const void*)g_weights);
-  float loss_acc = 0.f;
   for (int64_t ray = warp0; ray < R; ray += nwarps) {
     const float dx = rays_d[ray * 3 + 0], dy = rays_d[ray * 3 + 1], dz = rays_d[ray * 3 + 2];
     const float dnorm = sqrtf(dx * dx + dy * dy + dz * dz);
@@ -525,9 +517,8 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
       const float er = sr + bg - target[ray * 3 + 0], eg = sg + bg - target[ray * 3 + 1], eb = sb + bg - target[ray * 3 + 2];
       gr = 2.0f * er * loss_scale; gg = 2.0f * eg * loss_scale; gb = 2.0f * eb * loss_scale;
       gd = 0.f; ga = 0.f;
-      if (lane == 0) {
-        if (rgb_out != nullptr) { rgb_out[ray * 3 + 0] = sr + bg; rgb_out[ray * 3 + 1] = sg + bg; rgb_out[ray * 3 + 2] = sb + bg; }
-        loss_acc += (er * er + eg * eg + eb * eb) * loss_scale;
+      if (lane == 0 && rgb_out != nullptr) {
+        rgb_out[ray * 3 + 0] = sr + bg; rgb_out[ray * 3 + 1] = sg + bg; rgb_out[ray * 3 + 2] = sb + bg;
       }
     } else {
       gr = g_rgb ? g_rgb[ray * 3 + 0] : 0.f; gg = g_rgb ? g_rgb[ray * 3 + 1] : 0.f; gb = g_rgb ? g_rgb[ray * 3 + 2] : 0.f;
@@ -615,10 +606,6 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
       carryU = b0 + a0 * carryU;
     }
     __syncwarp();
-  }
-  if constexpr (TRAIN) {
-    loss_acc = warp_sum(loss_acc);
-    if (lane == 0 && loss_acc != 0.f) atomicAdd(loss, loss_acc);
   }
 }
 
@@ -713,15 +700,39 @@ extern "C" int ctx_composite_bwd(const float* raw, const float* z_vals, const fl
   CTX_RETURN_LAST();
 }
 
-// Fused training form of raw2outputs: forward + img2mse(rgb_map, target) + backward in one pass (see the kernel).
-// loss_scale = 1 / (3 R) for the mean over the rgb image; loss[0] is ADDED to (zero it once per step: the coarse and
-// the fine pass accumulate into the same scalar).  weights / rgb_map are optional outputs.
+namespace ctx {
+// loss[0] += loss_scale * sum over rays of |rgb - target|^2: one block, every thread a fixed strided set of rays, then
+// a fixed reduction tree, so the loss is the same on every run (atomics from many blocks would sum in arrival order).
+__global__ void __launch_bounds__(1024) loss_sum_kernel(const float* __restrict__ rgb, const float* __restrict__ target,
+                                                        int64_t R, float loss_scale, float* __restrict__ loss) {
+  __shared__ float s_part[32];
+  float acc = 0.f;
+  for (int64_t r = threadIdx.x; r < R; r += blockDim.x) {
+    const float er = rgb[r * 3 + 0] - target[r * 3 + 0], eg = rgb[r * 3 + 1] - target[r * 3 + 1],
+                eb = rgb[r * 3 + 2] - target[r * 3 + 2];
+    acc += (er * er + eg * eg + eb * eb) * loss_scale;
+  }
+  acc = warp_sum(acc);
+  if ((threadIdx.x & 31) == 0) s_part[threadIdx.x >> 5] = acc;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    acc = threadIdx.x < (blockDim.x >> 5) ? s_part[threadIdx.x] : 0.f;
+    acc = warp_sum(acc);
+    if (threadIdx.x == 0) loss[0] += acc;
+  }
+}
+}  // namespace ctx
+
+// Fused training form of raw2outputs: forward + img2mse(rgb_map, target) + backward in one pass (see the kernel),
+// then the loss from rgb_map (loss_sum_kernel).  loss_scale = 1 / (3 R) for the mean over the rgb image; loss[0] is
+// ADDED to (zero it once per step: the coarse and the fine pass accumulate into the same scalar).  weights is an
+// optional output.
 extern "C" int ctx_composite_train(const float* raw, const float* z_vals, const float* rays_d, const float* noise,
                                    int64_t R, int S, int white_bkgd, const float* target, float loss_scale,
                                    float* loss, float* g_raw, float* weights, float* rgb_map, void* stream) {
   if (R < 0 || S < 1 || S > 256 * ctx::kCompMaxChunks) return CTX_ERR_BAD_ARG;
   if (R == 0) return 0;
-  if (!raw || !z_vals || !rays_d || !target || !loss || !g_raw) return CTX_ERR_BAD_ARG;
+  if (!raw || !z_vals || !rays_d || !target || !loss || !g_raw || !rgb_map) return CTX_ERR_BAD_ARG;
   if (reinterpret_cast<uintptr_t>(raw) % 16 != 0 || reinterpret_cast<uintptr_t>(g_raw) % 16 != 0)
     return CTX_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
@@ -729,11 +740,12 @@ extern "C" int ctx_composite_train(const float* raw, const float* z_vals, const 
   if (S > ctx::comp_single_pass_max()) {
     ctx::composite_chunked_bwd_kernel<8, true><<<grid, block, 0, st>>>(
         (const float4*)raw, z_vals, rays_d, noise, R, S, white_bkgd, nullptr, nullptr, nullptr, nullptr, nullptr,
-        (float4*)g_raw, target, loss_scale, loss, weights, rgb_map);
-    CTX_RETURN_LAST();
+        (float4*)g_raw, target, loss_scale, nullptr, weights, rgb_map);
+  } else {
+    const int vec = ctx::comp_vec(S, {z_vals, noise, weights});
+    CTX_COMP_DISPATCH_BWD(true, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, nullptr, nullptr,
+                          nullptr, nullptr, nullptr, (float4*)g_raw, target, loss_scale, nullptr, weights, rgb_map)
   }
-  const int vec = ctx::comp_vec(S, {z_vals, noise, weights});
-  CTX_COMP_DISPATCH_BWD(true, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, nullptr, nullptr,
-                        nullptr, nullptr, nullptr, (float4*)g_raw, target, loss_scale, loss, weights, rgb_map)
+  ctx::loss_sum_kernel<<<1, 1024, 0, st>>>(rgb_map, target, R, loss_scale, loss);
   CTX_RETURN_LAST();
 }

@@ -4,9 +4,11 @@
 //   inputs in the activation records.  wgrad: dW = dZ^T * A summed over all points -- a split-K GEMM whose
 //   K dimension is the point index.  Both operands are [points x features] tile images consumed as
 //   MN-major operands, so no transposition pass exists anywhere.  Each CTA owns one (layer, segment) job
-//   and a slice of the point tiles, accumulates in TMEM, and flushes with fp32 red.global.add into the
-//   flat gradient bucket; bias gradients are column sums of dZ taken from the shared-memory tile while
-//   the MMAs run.  The kernel is HBM-bound (1 KB read per point per layer).
+//   and a slice of the point tiles, accumulates in TMEM, and stores its partial sums to scratch; bias
+//   gradients are column sums of dZ taken from the shared-memory tile while the MMAs run.  A second
+//   kernel adds the partials of each job in CTA order into the gradients, so that they are the same on
+//   every run (fp32 atomics would sum in arrival order).  The kernel is HBM-bound (1 KB read per point
+//   per layer).
 //
 // Gradients flow to the parameters only (the encoded inputs are data).
 // Reference semantics: autograd through NeRF2D.forward,
@@ -44,6 +46,8 @@ struct WgJob {
   int m_valid, n_lo, n_hi;
   float* bias_out; int bias_from_b; int bias_lo, bias_hi;   // column sums of the dZ operand -> bias_out[c - bias_lo]
   int cta_begin, cta_count;
+  float* part;        // per-CTA partials [cta][n - n_lo][m] (m < m_valid), then the bias partials [cta][c - bias_lo]
+  int64_t red_begin;  // first element of this job in the reduction's index space
 };
 struct WgradArgs {
   int n_jobs;
@@ -176,8 +180,9 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_kernel(const __grid_c
         const int c = cw + ci * 4;
         if (c < n_chunks && lane < 4 && my_tiles > 0) {
           const int ch = c * 8 + lane * 2;
-          if (ch >= J.bias_lo && ch < J.bias_hi) atomicAdd(J.bias_out + ch - J.bias_lo, lo);
-          if (ch + 1 >= J.bias_lo && ch + 1 < J.bias_hi) atomicAdd(J.bias_out + ch + 1 - J.bias_lo, hi);
+          float* bp = J.part + (size_t)cta_count * (J.n_hi - J.n_lo) * J.m_valid + (size_t)split * (J.bias_hi - J.bias_lo);
+          if (ch >= J.bias_lo && ch < J.bias_hi) bp[ch - J.bias_lo] = lo;
+          if (ch + 1 >= J.bias_lo && ch + 1 < J.bias_hi) bp[ch + 1 - J.bias_lo] = hi;
         }
       }
     }
@@ -186,8 +191,8 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_kernel(const __grid_c
       tc::mbar_wait(&ctl->done, 0);
       tc::tc_fence_after();
       const int q = warp & 3;
-      const int n_lo = J.n_lo, n_hi = J.n_hi, ld_out = J.ld_out, col_off = J.col_off, transposed = J.transposed;
-      float* const outp = J.out;
+      const int n_lo = J.n_lo, n_hi = J.n_hi, m_valid = J.m_valid;
+      float* const outp = J.part + (size_t)split * (n_hi - n_lo) * m_valid;
       for (int mh = 0; mh < m_halves; ++mh) {
         const int m = mh * 128 + q * 32 + lane;
         for (int cb = 0; cb < (b_ch + 31) / 32; ++cb) {
@@ -207,15 +212,11 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_kernel(const __grid_c
             for (int j = 16; j < 32; ++j) vr[j] = 0u;
           }
           tc::tmem_wait_ld(vr);
-          if (m < J.m_valid) {
+          if (m < m_valid) {
 #pragma unroll
             for (int j = 0; j < 32; ++j) {
               const int n = cb * 32 + j;
-              if (n >= n_lo && n < n_hi) {
-                float* dst = transposed ? (outp + (size_t)(n - n_lo) * ld_out + col_off + m)
-                                        : (outp + (size_t)m * ld_out + col_off + (n - n_lo));
-                atomicAdd(dst, __uint_as_float(vr[j]));
-              }
+              if (n >= n_lo && n < n_hi) outp[(size_t)(n - n_lo) * m_valid + m] = __uint_as_float(vr[j]);
             }
           }
         }
@@ -230,6 +231,36 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_kernel(const __grid_c
   }
 }
 
+// Sums the partials of every job over its CTAs, in CTA order, into the gradients (one thread per gradient element:
+// the jobs write disjoint elements, so the result does not depend on the schedule).
+__global__ void __launch_bounds__(256) wgrad_reduce_kernel(const __grid_constant__ WgradArgs a, int64_t n_elems) {
+  for (int64_t e = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; e < n_elems; e += (int64_t)gridDim.x * blockDim.x) {
+    int ji = 0;
+    for (int j = 1; j < a.n_jobs; ++j)
+      if (e >= a.job[j].red_begin) ji = j;
+    const WgJob& J = a.job[ji];
+    const int64_t k = e - J.red_begin;
+    const int64_t nw = (int64_t)(J.n_hi - J.n_lo) * J.m_valid;
+    const int nc = (int)(J.cta_count < a.n_tiles ? J.cta_count : a.n_tiles);
+    float acc = 0.f;
+    if (k < nw) {
+      for (int s = 0; s < nc; ++s) acc += J.part[s * nw + k];
+      const int n = (int)(k / J.m_valid), m = (int)(k % J.m_valid);
+      float* dst = J.transposed ? (J.out + (size_t)n * J.ld_out + J.col_off + m)
+                                : (J.out + (size_t)m * J.ld_out + J.col_off + n);
+      *dst += acc;
+    } else {
+      const int nb = J.bias_hi - J.bias_lo, b = (int)(k - nw);
+      const float* bp = J.part + (size_t)J.cta_count * nw;
+      for (int s = 0; s < nc; ++s) acc += bp[s * nb + b];
+      J.bias_out[b] += acc;
+    }
+  }
+}
+
+// Scratch of the per-CTA partials: at most kNumSMs CTAs, each with at most a 256 x 256 block and 256 bias sums.
+constexpr int64_t kWgPartFloats = (int64_t)kNumSMs * (256 * 256 + 256);
+
 // ---------------------------------------------------------------------------------------------------------
 // View-direction head without a feature-layer record.  feature = W_f h + b_f is linear (no activation,
 // reference comment block src/run_nerf_helpers.py:119-121), v = relu(W_vh feature + W_vd x_d + b_v).  With
@@ -241,7 +272,7 @@ __global__ void __launch_bounds__(kWgThreads, 1) mlp_wgrad_kernel(const __grid_c
 //     dw_alpha = G[:, 128+3]      db_alpha = s[128+3]
 // (W_vh, W_f, b_f as the kernels see them: rounded to bf16).  So neither the feature activations nor dZ_feature are
 // ever written to HBM, and the two 1 KB-per-point jobs that read them are replaced by one 800 B-per-point job.
-// scratch: Gt [144][256] (n-major) followed by s [144], fp32, zeroed by the launcher.
+// scratch: Gt [144][256] (n-major) followed by s [144], fp32, zeroed by the launcher; the wgrad partials follow.
 constexpr int kPostGtFloats = 144 * 256, kPostScratchFloats = 144 * 256 + 144;
 __device__ __forceinline__ float bf16r(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
 
@@ -325,23 +356,23 @@ __global__ void __launch_bounds__(256) wgrad_post_kernel(
 // grads: HOST array of DEVICE pointers in the order of ctx_mlp_pack's `params`
 // (gradients are ACCUMULATED into them: zero them first for a fresh gradient).
 // params: the fp32 parameters themselves, same order (the view-direction head rebuilds the gradients of
-// feature_linear / views_linears.0[:, :256] from G and the weights, see wgrad_post_kernel); scratch: device buffer of
-// ctx_mlp_wgrad_scratch_floats() floats (both only used with a view-direction net; may be null otherwise).
+// feature_linear / views_linears.0[:, :256] from G and the weights, see wgrad_post_kernel; only used with a
+// view-direction net, may be null otherwise); scratch: device buffer of ctx_mlp_wgrad_scratch_floats() floats.
 // max_sms > 0: use at most that many CTAs (rounded down to even) and launch them as 2-CTA clusters, so that they
 // pack into whole SM pairs and a concurrent cluster kernel (dgrad of the other network) finds free pairs.
-extern "C" int ctx_mlp_wgrad_scratch_floats(void) { return ctx::kPostScratchFloats; }
+extern "C" int ctx_mlp_wgrad_scratch_floats(void) { return (int)(ctx::kPostScratchFloats + ctx::kWgPartFloats); }
 
 extern "C" int ctx_mlp_wgrad_ex(const void* net_host, const void* acts, const void* dacts, int64_t P,
                                 float* const* grads, int n_grads, const float* const* params, float* scratch,
                                 int max_sms, void* stream) {
   if (P < 0) return CTX_ERR_BAD_ARG;
   if (P == 0) return 0;
-  if (!net_host || !acts || !dacts || !grads) return CTX_ERR_BAD_ARG;
+  if (!net_host || !acts || !dacts || !grads || !scratch) return CTX_ERR_BAD_ARG;
   const CtxMlpNet& net = *reinterpret_cast<const CtxMlpNet*>(net_host);
   const bool views = net.in_views > 0;
   const int D = views ? net.n_layers - 2 : net.n_layers;
   if (n_grads != 2 * D + (views ? 8 : 2)) return CTX_ERR_BAD_ARG;
-  if (views && (!params || !scratch)) return CTX_ERR_BAD_ARG;
+  if (views && !params) return CTX_ERR_BAD_ARG;
   cudaStream_t st = (cudaStream_t)stream;
   static ctx::DeviceOnce attr_once;
   if (attr_once.needed()) {
@@ -438,7 +469,17 @@ extern "C" int ctx_mlp_wgrad_ex(const void* net_host, const void* acts, const vo
       const int k = j % nj;
       if (cost[k] >= 384.f && (int64_t)given[k] < n_tiles) { ++given[k]; ++used; }
     }
-    for (int j = 0; j < nj; ++j) { w.job[j].cta_begin = begin; w.job[j].cta_count = given[j]; begin += given[j]; }
+    float* part = scratch + ctx::kPostScratchFloats;
+    int64_t red = 0;
+    for (int j = 0; j < nj; ++j) {
+      ctx::WgJob& J = w.job[j];
+      J.cta_begin = begin; J.cta_count = given[j]; begin += given[j];
+      if (!J.bias_out) J.bias_lo = J.bias_hi = 0;
+      const int64_t per_cta = (int64_t)(J.n_hi - J.n_lo) * J.m_valid + (J.bias_hi - J.bias_lo);
+      J.part = part; part += per_cta * given[j];
+      J.red_begin = red; red += per_cta;
+    }
+    if (part > scratch + ctx::kPostScratchFloats + ctx::kWgPartFloats) return CTX_ERR_UNSUPPORTED;
     w.n_jobs = nj;
     if (capped && (begin & 1) == 0) {
       cudaLaunchConfig_t cfg = {};
@@ -453,6 +494,7 @@ extern "C" int ctx_mlp_wgrad_ex(const void* net_host, const void* acts, const vo
     } else {
       ctx::mlp_wgrad_kernel<<<begin, ctx::kWgThreads, ctx::kWgSmemBytes, st>>>(w);
     }
+    ctx::wgrad_reduce_kernel<<<2 * budget, 256, 0, st>>>(w, red);
   }
   {
     cudaError_t e = cudaGetLastError();

@@ -37,7 +37,8 @@ def mlp_dgrad(module, packed, acts, P, g_out, max_sms=0):
 
 
 def wgrad_scratch(dev):
-    """fp32 scratch of the view-direction head's G job (ctx_mlp_wgrad_scratch_floats floats; zeroed by the launcher)."""
+    """fp32 scratch of the wgrad kernels (ctx_mlp_wgrad_scratch_floats floats): the per-CTA partial sums and the
+    view-direction head's G job."""
     from . import _lib
     return torch.empty(_lib.lib().ctx_mlp_wgrad_scratch_floats(), device=dev, dtype=torch.float32)
 
@@ -49,7 +50,7 @@ def mlp_wgrad(module, acts, dacts, P, sinks=None, max_sms=0, scratch=None):
     grads, params = _grad_targets(module, sinks, dev)
     arr = (ctypes.c_void_p * len(grads))(*[t.data_ptr() for t in grads])
     parr = (ctypes.c_void_p * len(params))(*[t.data_ptr() for t in params])
-    if scratch is None and module._desc.in_views > 0:
+    if scratch is None:
         scratch = wgrad_scratch(dev)
     with torch.cuda.device(dev):
         call("ctx_mlp_wgrad_ex", module._desc.p, ptr(acts), ptr(dacts), P, ctypes.cast(arr, ctypes.c_void_p),

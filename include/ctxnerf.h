@@ -106,8 +106,9 @@ int ctx_resample_bwd(const float* bins, int64_t bins_stride, int mid_bins, const
 /* Fused training form of raw2outputs (NerfTrainer.step): forward + img2mse(rgb_map, target)
  * (src/run_nerf_helpers.py:9) + backward in ONE pass over raw.  g_raw [R,S,4] = d loss / d raw with
  * loss = sum((rgb_map - target)^2) * loss_scale (loss_scale = 1/(3R) for the image mean); loss[0] += that value
- * (zero it once per step; the coarse and the fine pass add into the same scalar).  weights [R,S] and rgb_map [R,3]
- * are optional outputs (the coarse pass feeds sample_pdf with its weights).                        */
+ * (zero it once per step; the coarse and the fine pass add into the same scalar), summed from rgb_map [R,3] in a
+ * fixed order so that it is the same on every run.  weights [R,S] is an optional output (the coarse pass feeds
+ * sample_pdf with its weights).                                                                    */
 int ctx_composite_train(const float* raw, const float* z_vals, const float* rays_d, const float* noise,
                         int64_t R, int S, int white_bkgd, const float* target, float loss_scale, float* loss,
                         float* g_raw, float* weights, float* rgb_map, void* stream);
@@ -161,11 +162,12 @@ int ctx_mlp_bwd(const void* net, const void* wtpacked, const float* fparams, con
  * dgrad fills the dZ records from g_out, wgrad reduces records + dZ records into the gradients. */
 int ctx_mlp_dgrad(const void* net, const void* wtpacked, const float* fparams, const float* g_out,
                   const void* acts, void* dacts, int64_t P, void* stream);
-/* params (HOST array of DEVICE pointers, order of ctx_mlp_pack) and scratch (device,
- * ctx_mlp_wgrad_scratch_floats() floats, zeroed by the launcher) are read only for a view-direction net: the
- * feature layer is linear, so its weight gradients and those of views_linears.0[:, :256] are rebuilt from
- * G = [dZ_views | g_out]^T h and the weights instead of from records of the feature activations (which are never
- * written).  Both may be NULL for a net without views.                                                        */
+/* scratch (device, ctx_mlp_wgrad_scratch_floats() floats) holds the per-CTA partial sums, which a second kernel
+ * adds in a fixed order, so the gradients are the same on every run.  params (HOST array of DEVICE pointers, order
+ * of ctx_mlp_pack) are read only for a view-direction net, and may be NULL for a net without views: the feature
+ * layer is linear, so its weight gradients and those of views_linears.0[:, :256] are rebuilt from
+ * G = [dZ_views | g_out]^T h (in scratch) and the weights instead of from records of the feature activations
+ * (which are never written).                                                                                    */
 int ctx_mlp_wgrad_scratch_floats(void);
 int ctx_mlp_wgrad(const void* net, const void* acts, const void* dacts, int64_t P, float* const* grads,
                   int n_grads, const float* const* params, float* scratch, void* stream);

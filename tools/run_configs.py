@@ -62,9 +62,10 @@ for lr in (12, 14, 16, 18, 20, 22):
         # g_raw 16S + weights 4S
         tgt = torch.rand(R, 3, device=dev); g_raw = torch.empty_like(raw); wts = torch.empty(R, S, device=dev)
         loss = torch.zeros(1, device=dev)
+        rgb = torch.empty(R, 3, device=dev)
         from ctxnerf._lib import call, ptr, stream_ptr
         t = timeit(lambda: call("ctx_composite_train", ptr(raw), ptr(z), ptr(d), None, R, S, 1, ptr(tgt), 1.0 / (3 * R),
-                                ptr(loss), ptr(g_raw), ptr(wts), None, stream_ptr(dev)), iters=3, warm=1)
+                                ptr(loss), ptr(g_raw), ptr(wts), ptr(rgb), stream_ptr(dev)), iters=3, warm=1)
         row["composite_train_gbs"] = R * (40 * S + 24) / t / 1e9
         # separate backward (all five output gradients given): reads raw 16S + z 4S + g_weights 4S + 36, writes g_raw 16S
         g = [torch.randn(R, 3, device=dev), torch.randn(R, device=dev), torch.randn(R, device=dev),
