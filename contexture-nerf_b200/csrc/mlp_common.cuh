@@ -10,7 +10,7 @@
 
 namespace ctx {
 
-// Tensor map over a record buffer for the epilogues' tile stores: a [128 points x 256 channels] bf16 tile sits in
+// Tensor map over a record buffer for the dgrad epilogue's tile stores: a [128 points x 256 channels] bf16 tile sits in
 // shared memory as [k8 = 32][half = 2][64 rows x 16 B] (the K-major A-operand image) and in the record as two
 // 64-point halves of [k8][64 rows x 16 B]; with 8-byte elements that is the 4-D box {128, 2, 32, 1} of the tensor
 //   dim0: 128 x u64 (1 KB, contiguous) | dim1: half, stride 32 KB | dim2: 1 KB units of a tile's record, stride 1 KB
@@ -58,8 +58,6 @@ struct MlpFwdArgs {
   unsigned long long* prof; // nullable: per-CTA cycle counters (diagnostics), 16 per CTA
   unsigned long long* hang; // nullable: host-visible buffer for the deadlock reporter (diagnostics)
   int debug;                // diagnostics: 1 = epilogue skips TMEM loads/stores, 2 = issuer skips the MMAs
-  int use_tma;              // training: 256-wide activation tiles leave through one tensor-map TMA store each
-  CUtensorMap tmap;         // over the activation record buffer (make_record_tensor_map)
 };
 
 
@@ -99,14 +97,10 @@ __device__ __forceinline__ void store_row8(uint8_t* tile, int row, int ch0, cons
     q.x = pack_bf16x2(v[0], v[1]); q.y = pack_bf16x2(v[2], v[3]);
     q.z = pack_bf16x2(v[4], v[5]); q.w = pack_bf16x2(v[6], v[7]);
   }
-#ifndef CTX_X_NO_STS      // (timing experiments only: tools/build_variants.sh)
   if (tile) *reinterpret_cast<uint4*>(tile + (ch0 >> 3) * kK8Stride + (row >> 3) * 128 + (row & 7) * 16) = q;
-#endif
-#ifndef CTX_X_NO_STG
   if (gtile)   // streaming store: the record is next read by another kernel, keep it out of the (small) L1
     __stcs(reinterpret_cast<uint4*>(gtile + (row >> 6) * (gC * 128) + (ch0 >> 3) * 1024 + ((row & 63) >> 3) * 128 +
                                     (row & 7) * 16), q);
-#endif
 }
 
 }  // namespace ctx

@@ -15,7 +15,7 @@
 #include <stdlib.h>
 #include <string.h>
 
-#ifdef CTX_DG_PROF      // variant build (tools/build_variants.sh): per-role cycle counters, 16 x uint64 per CTA
+#ifdef CTXNERF_DIAG     // diagnostics build (include/ctxnerf_diag.h): per-role cycle counters, 16 x uint64 per CTA
 static unsigned long long* g_dg_prof = nullptr;
 extern "C" int ctx_dgrad_set_prof(void* p) { g_dg_prof = (unsigned long long*)p; return 0; }
 #define DGCLK() clock64()
@@ -41,7 +41,7 @@ struct DgradArgs {
   int n_steps;
   int step_src[CTX_MLP_MAX_LAYERS];
   int step_dst[CTX_MLP_MAX_LAYERS];
-  unsigned long long* prof;  // variant builds only
+  unsigned long long* prof;  // diagnostics build only
   int use_tma;               // dZ tiles of the inner steps leave through one tensor-map TMA store per tile-layer
   CUtensorMap tmap;          // over the dZ record buffer (mlp_common.cuh: make_record_tensor_map)
 };
@@ -184,7 +184,7 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
             }
           }
         }
-#ifdef CTX_DG_PROF
+#ifdef CTXNERF_DIAG
         if (a.prof) { unsigned long long* pp = a.prof + blockIdx.x * 16 + ph * 3; pp[0] = t_act; pp[1] = t_full; pp[2] = DGCLK() - t_beg; }
 #endif
       }
@@ -219,7 +219,7 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
     }
     if (tc::elect_one()) tc::bulk_wait<0>();
     __syncwarp();
-#ifdef CTX_DG_PROF
+#ifdef CTXNERF_DIAG
     if (a.prof && lane == 0) { a.prof[blockIdx.x * 16 + 6] = t_rdy; a.prof[blockIdx.x * 16 + 7] = t_rd; }
 #endif
   }
@@ -372,15 +372,6 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
               for (int j = 0; j < 32; j += 8)
                 store_row8(NEXT ? my_h : nullptr, row, cb * 32 + j, v + j, false, grec, 256);
             };
-#ifdef CTX_X_SERIAL_LD
-            uint32_t va[32];
-#pragma unroll
-            for (int cbi = 0; cbi < 4; ++cbi) {
-              tc::tmem_ld32(my_acc + cbi * 32, va);
-              tc::tmem_wait_ld(va);
-              process(va, cbi);
-            }
-#else
             // the load of block c+1 is in flight while block c is processed (two register buffers; affordable since
             // the epilogue warps own 224 registers)
             uint32_t va[32], vb[32];
@@ -396,7 +387,6 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
             process(va, 2);
             tc::tmem_wait_ld(vb);
             process(vb, 3);
-#endif
           };
           {
             using std::integral_constant;
@@ -423,7 +413,7 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
         }
       }
     }
-#ifdef CTX_DG_PROF
+#ifdef CTXNERF_DIAG
     if (a.prof && lane == 0 && (warp == 4 || warp == 11)) {
       unsigned long long* pp = a.prof + blockIdx.x * 16 + (warp == 4 ? 8 : 12);
       pp[0] = t_acc; pp[1] = t_free; pp[2] = t_body; pp[3] = warp == 4 ? (unsigned long long)(DGCLK() - t_beg) : (unsigned long long)t_head;
@@ -431,11 +421,6 @@ mlp_dgrad_kernel(const __grid_constant__ DgradArgs a) {
 #endif
   }
 
-#ifdef CTX_DG_PROF
-  if (a.prof && warp == 4 && lane == 0) {
-    // (written by one epilogue warp: the counters live in that branch; see the macro below)
-  }
-#endif
   tc::tc_fence_before();
   tc::cluster_sync_all();
   if (warp == 1) {
@@ -461,7 +446,7 @@ int ctx_launch_dgrad(const CtxMlpNet& net, const void* wtpacked, const float* fp
     // when the driver cannot encode the map)
     static const bool want = [] { const char* e = getenv("CTXNERF_DGRAD_TMA"); return !(e && e[0] == '0'); }();
     const int64_t n_tiles = 4 * ctx::ceil_div(P, (int64_t)ctx::kTileM * 4);
-#ifdef CTX_DG_PROF
+#ifdef CTXNERF_DIAG
     a.prof = g_dg_prof;
 #else
     a.prof = nullptr;

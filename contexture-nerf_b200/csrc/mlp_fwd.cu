@@ -30,8 +30,6 @@
 // Reference semantics: NeRF2D.forward, /root/reference/src/run_nerf_helpers.py:106-135
 // (+ commented view branch :117-127); Embedder.embed :44-45.
 #include "mlp_common.cuh"
-#include <stdlib.h>
-#include <string.h>
 
 namespace ctx {
 
@@ -39,7 +37,8 @@ namespace ctx {
 // quarter, 104 registers) -- training forward 0.95 -> 1.01 ms; eight warps on 16-column blocks -- 0.950 -> 0.966 ms:
 // the epilogue is not latency-bound per warp.  A setmaxnreg split must hand out exactly what the CTA was launched with
 // (4 x 56 + 8 x 224 = 12 x 168 here): setmaxnreg.inc only draws on registers the CTA itself released, and a split
-// that asks for more (4 x 56 + 16 x 112 > 20 x 96) hangs the kernel.
+// that asks for more (4 x 56 + 16 x 112 > 20 x 96) hangs the kernel.  Shipping each finished activation tile to its
+// record with one TMA tensor store from a store warp, instead of the epilogue's register stores: 0.95 -> 1.14 ms.
 constexpr int kStages2 = 8;          // 8 KB half-chunk stages, handled in PAIRS (one full/empty barrier per pair)
 constexpr int kPairs2 = kStages2 / 2;
 constexpr int kHeadFloats = 648;    // view-direction head block staged in shared memory (w_alpha, W_rgb, biases)
@@ -48,7 +47,6 @@ constexpr int kStage2Bytes = kStageBytes / 2;   // 8 KB half-chunk
 struct __align__(8) Mlp2SmemCtl {
   uint64_t full[kPairs2], empty[kPairs2];
   uint64_t acc_full[kTiles], act_ready[kTiles];
-  uint64_t rec_ready[kTiles], rec_free[kTiles];   // epilogue -> store warp: tile written ; store warp -> epilogue: read
   uint32_t tmem_base;
 };
 constexpr size_t kMlp2SmemBytes = (size_t)kTiles * (kHBytes + kXBytes) + (size_t)kStages2 * kStage2Bytes +
@@ -141,7 +139,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
     }
     for (int t = 0; t < kTiles; ++t) {
       tc::mbar_init(&ctl->acc_full[t], 1); tc::mbar_init(&ctl->act_ready[t], 16);
-      tc::mbar_init(&ctl->rec_ready[t], 8); tc::mbar_init(&ctl->rec_free[t], 1);
     }
     tc::mbar_fence_init();
   }
@@ -287,33 +284,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
         }
       }
     }
-  } else if (warp == 3 && kRec && a.use_tma) {
-    // ============ record-store warp (training): one TMA tensor store per finished 256-wide activation tile ============
-    // The epilogue leaves the tile in shared memory anyway (next layer's A operand); this warp ships the same bytes
-    // to the activation record with ONE instruction, so the epilogue warps issue no global stores for it.
-    uint32_t n_st = 0;
-    for (int64_t it = cid; it < n_citers; it += ncl) {
-      for (int l = 0; l < net.n_layers; ++l) {
-        const int Lact = net.L[l].act_slot;
-        if (Lact < 0 || net.L[l].rec_ch != CTX_MLP_W || net.L[l].epi == CTX_EPI_FINAL_VIEWS ||
-            net.L[l].epi == CTX_EPI_FINAL_OUT)
-          continue;
-#pragma unroll
-        for (int ph = 0; ph < 2; ++ph) {
-          tc::mbar_wait(&ctl->rec_ready[ph], n_st & 1);
-          if (tc::elect_one()) {
-            tc::tma_store_4d(&a.tmap, h_buf + ph * kHBytes, 0, 0, Lact >> 10, (int)(it * 4 + ph * 2 + r));
-            tc::bulk_commit();
-            tc::bulk_wait_read<0>();          // the tile may be overwritten once the copy has read it
-            tc::mbar_arrive(&ctl->rec_free[ph]);
-          }
-          __syncwarp();
-        }
-        ++n_st;
-      }
-    }
-    if (tc::elect_one()) tc::bulk_wait<0>();
-    __syncwarp();
   }
   } else {
     reg_alloc<kEpiRegs>();
@@ -331,22 +301,14 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
     long long t_acc = 0, t_body = 0, t_enc = 0;
     const long long t_begin = PCLK();
 
-    const bool use_tma = kRec && a.use_tma != 0;
-    uint32_t n_st0 = 0, n_st1 = 0;          // TMA stores issued so far from each tile buffer
-    auto arrive_act = [&](int ph, bool rec = false) {
+    auto arrive_act = [&](int ph) {
       tc::fence_proxy_async_smem();
       tc::tc_fence_before();
       __syncwarp();
       if (lane == 0) {
-        if (rec) tc::mbar_arrive(&ctl->rec_ready[ph]);
         if (r == 0) tc::mbar_arrive(&ctl->act_ready[ph]);
         else tc::mbar_arrive_remote(&ctl->act_ready[ph], 0);
       }
-    };
-    // before (re)writing a tile's h buffer: the last TMA store issued from it must have finished reading it
-    auto wait_tile_free = [&](int ph) {
-      const uint32_t n = ph ? n_st1 : n_st0;
-      if (n > 0) tc::mbar_wait(&ctl->rec_free[ph], (n - 1) & 1);
     };
     auto encode_tile = [&](int64_t it, int te) {   // encode rows of tile `te` for cluster iteration `it`
       const int64_t tile_idx = it * 4 + te * 2 + r;
@@ -424,8 +386,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
           acc_phase[ph] ^= 1;
           tc::tc_fence_after();
           float head[4] = {0.f, 0.f, 0.f, 0.f};
-          const bool tma_rec = use_tma && !is_final && Lact >= 0 && Lrec == CTX_MLP_W;
-          if (kRec && !is_final) wait_tile_free(ph);
           // The bias is already inside the accumulator (constant-1 channel x bias row of the weight stream),
           // so a hidden-layer epilogue is: TMEM load -> (training: sign mask) -> relu+bf16 pack -> store.
           // One straight-line instantiation per (epilogue kind, relu): the per-block path of a plain hidden
@@ -434,10 +394,8 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
             constexpr int EPI = decltype(epi_c)::value;
             constexpr bool RELU = decltype(relu_c)::value;
             constexpr bool FINAL = (EPI == CTX_EPI_FINAL_VIEWS || EPI == CTX_EPI_FINAL_OUT);
-            // (feature layer: no record; tma_rec: the tile leaves through the store warp)
-            uint8_t* const grec = (kRec && Lact >= 0 && !tma_rec) ? rec + Lact : nullptr;
+            uint8_t* const grec = (kRec && Lact >= 0) ? rec + Lact : nullptr;   // (feature layer: no record)
             auto process = [&](const uint32_t (&vr)[32], int cb) {
-#ifndef CTX_X_NO_MASK
               if constexpr (kRec && RELU) {
                 // bit (31-j) = sign of pre-activation j (the ReLU mask the dgrad kernel reads); four independent
                 // shift chains instead of one 32-deep dependent one
@@ -452,7 +410,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
                 const uint32_t neg = (n0 << 24) | (n1 << 16) | (n2 << 8) | n3;
                                 __stcs(reinterpret_cast<uint32_t*>(rec + Lmask) + cb * kTileM + row, neg);   // [column block][row]: coalesced
               }
-#endif
               float v[32];
 #pragma unroll
               for (int j = 0; j < 32; ++j) v[j] = __uint_as_float(vr[j]);
@@ -485,7 +442,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
               }
             };
             const int cb0 = hi * ncb;
-#ifndef CTX_X_PIPE_LD
             // (loads are NOT run ahead of the processing: measured slower in this kernel, before and after the
             //  epilogue warps got 224 registers; the dgrad epilogue does profit from it)
             uint32_t va[32];
@@ -494,19 +450,6 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
               tc::tmem_wait_ld(va);
               process(va, cb0 + cbi);
             }
-#else
-            uint32_t va[32], vb[32];
-            tc::tmem_ld32(my_acc + cb0 * 32, va);
-            tc::tmem_wait_ld(va);
-            for (int cbi = 0; cbi < ncb; cbi += 2) {
-              tc::tmem_ld32(my_acc + (cb0 + cbi + 1) * 32, vb);
-              process(va, cb0 + cbi);
-              tc::tmem_wait_ld(vb);
-              if (cbi + 2 < ncb) tc::tmem_ld32(my_acc + (cb0 + cbi + 2) * 32, va);
-              process(vb, cb0 + cbi + 1);
-              if (cbi + 2 < ncb) tc::tmem_wait_ld(va);
-            }
-#endif
           };
           if (!(dbg & 1)) {
             using std::integral_constant;
@@ -572,8 +515,7 @@ mlp_fwd_kernel(const __grid_constant__ MlpFwdArgs a) {
             t_enc += PCLK() - e2;
             if (nit < n_citers) arrive_act(ph);
           } else {
-            arrive_act(ph, tma_rec);
-            if (tma_rec) { if (ph) ++n_st1; else ++n_st0; }
+            arrive_act(ph);
           }
           t_body += PCLK() - e1;
         }
@@ -641,15 +583,6 @@ extern "C" int ctx_mlp_fwd_ex(const void* net_host, const void* wpacked, const f
   a.wpacked = (const uint8_t*)wpacked; a.fparams = fparams; a.mode = mode; a.x = x; a.x_ld = x_ld;
   a.rays_o = rays_o; a.rays_d = rays_d; a.viewdirs = viewdirs; a.z = z; a.S = S; a.L_pts = L_pts;
   a.L_dirs = L_dirs; a.P = P; a.out = out; a.acts = (uint8_t*)acts;
-  a.use_tma = 0;
-  memset(&a.tmap, 0, sizeof(a.tmap));
-  if (a.acts) {
-    // activation tiles can go out by TMA tensor stores (CTXNERF_FWD_TMA=1; default off: measured slower than the
-    // register stores in this kernel, unlike in dgrad -- profiles/README.md r02)
-    static const bool want = [] { const char* e = getenv("CTXNERF_FWD_TMA"); return e && e[0] == '1'; }();
-    const int64_t n_tiles = 4 * ctx::ceil_div(P, (int64_t)ctx::kTileM * 4);
-    a.use_tma = want && ctx::make_record_tensor_map(&a.tmap, a.acts, a.net.act_tile_bytes, n_tiles) == 0;
-  }
   a.prof = (unsigned long long*)ctx_mlp_prof_buffer; a.debug = ctx_mlp_debug_flags;
   a.hang = (unsigned long long*)ctx_mlp_hang_buffer;
   cudaStream_t st = (cudaStream_t)stream;

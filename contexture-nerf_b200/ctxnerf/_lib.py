@@ -11,7 +11,7 @@ import os
 from ctypes import c_char_p, c_float, c_int, c_int64, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("CTXNERF_LIB") or os.path.join(_HERE, "libctxnerf.so")   # override: kernel experiments
+LIB_PATH = os.path.join(_HERE, "libctxnerf.so")
 
 _lib = None
 
@@ -95,6 +95,7 @@ _DIAG_SIGNATURES = {
     "ctx_mlp_set_prof_buffer": (c_int, [P]),
     "ctx_mlp_set_debug": (c_int, [c_int]),
     "ctx_mlp_set_hang_buffer": (c_int, [P]),
+    "ctx_dgrad_set_prof": (c_int, [P]),
     "ctx_tcgen05_selftest": (c_int, [P, P, P, c_int, c_int, c_int, c_int, P]),
     "ctx_tcgen05_mma_rate": (c_int, [c_int, c_int, c_int, c_int, P, c_int, P, P]),
     "ctx_tcgen05_sync_cost": (c_int, [P, c_int, P]),

@@ -21,7 +21,7 @@ BUILD_DIR = os.path.join(CSRC, "build")
 LIB_PATH = os.path.join(PKG_DIR, "libctxnerf.so")
 DIAG_LIB_PATH = os.path.join(PKG_DIR, "libctxnerf_diag.so")   # diagnostics build (include/ctxnerf_diag.h)
 DIAG_DIR = os.path.join(CSRC, "diag")
-DIAG_VARIANT = {"mlp_fwd.cu"}     # product sources that carry #ifdef CTXNERF_DIAG sections
+DIAG_VARIANT = {"mlp_fwd.cu", "mlp_dgrad.cu"}     # product sources that carry #ifdef CTXNERF_DIAG sections
 
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr",

@@ -65,7 +65,6 @@ class _Plan:
         self.graph_tail = None     # second graph (Adam + re-pack) when the all-reduce runs between the two
         self.eager_steps = 0
         self.kernels_per_step = 0
-        self.fine_reduced = False  # the head has already all-reduced the fine network's half of the bucket
 
 
 class NerfTrainer:
@@ -100,13 +99,9 @@ class NerfTrainer:
         if self.world_size > 1 and os.environ.get("CTXNERF_NCCL", "1") != "0" and "nccl" in dist_backend():
             self.comm = self._make_comm(dev)
         self.reduce_gradients = True       # (tools/dist_check.py turns the exchange off for its single-process sums)
-        # CTXNERF_SPLIT_REDUCE=1: the bucket goes in two halves -- the fine network's right behind its wgrad, beside the
-        # coarse chain still running on the side stream, the coarse network's after the join.  Measured on 8 GPUs it is
-        # SLOWER than one whole-bucket call after the join (4.45 vs 4.39 ms: the early NCCL kernel waits for the slowest
-        # rank while holding SMs the coarse chain wants), so the default is the single call
-        # (profiles/r02/allreduce_routes_8gpu.txt)
-        self._n_coarse = sum(p.numel() for p in self.coarse.parameters())
-        self.split_reduce = self.comm is not None and os.environ.get("CTXNERF_SPLIT_REDUCE", "0") == "1"
+        # The bucket is all-reduced in one call after the join of the two backward chains.  bench.py reads this flag
+        # to name the route; a two-halves route measured slower and was removed (DESIGN.md §5), so it is always False.
+        self.split_reduce = False
         self._loss = torch.zeros(1, device=dev)
         # device-side step state: [0] Philox seed offset, [1] Adam step count (ctx_step_tick advances both)
         self._ctr = torch.zeros(2, device=dev, dtype=torch.int64)
@@ -123,21 +118,12 @@ class NerfTrainer:
         self._packed_version = -1
         self._plans = {}
         self.timers = None      # optional dict name -> list[(start_event, end_event)]; forces the eager path
-        n_sm = torch.cuda.get_device_properties(dev).multi_processor_count
-        self.n_sms = n_sm
+        self.n_sms = torch.cuda.get_device_properties(dev).multi_processor_count
         # Backward schedule: the two networks' chains are independent and their kernels bind on different resources
         # (dgrad: tensor pipe / epilogue; wgrad: HBM reads).  The coarse chain runs on a side stream inside an SM
         # budget while wgrad of the fine network streams its records through the other SMs.
         self.overlap_backward = os.environ.get("CTXNERF_OVERLAP", "1") != "0"
         self.side_sms = _env_int("CTXNERF_SIDE_SMS", 44)
-        # CTXNERF_EARLY_COARSE=1: start the coarse backward chain right after the coarse compositing (its loss term
-        # does not depend on the fine pass), beside resample + fwd_fine + dgrad_fine, which then take main_sms SMs
-        self.early_coarse = os.environ.get("CTXNERF_EARLY_COARSE", "0") == "1"
-        self.main_sms = _env_int("CTXNERF_MAIN_SMS", n_sm - self.side_sms)
-        # CTXNERF_SCHED=queue: both backward chains at full grid size on two streams, no SM budgets: the hardware hands
-        # an SM to the next kernel's CTA as soon as one of the running kernel's CTAs retires (no drain / fill bubble
-        # between launches); measured against the budgeted schedule in profiles/README.md
-        self.sched_queue = os.environ.get("CTXNERF_SCHED", "") == "queue"
         self.use_graph = os.environ.get("CTXNERF_GRAPH", "1") != "0"
         self._side = torch.cuda.Stream(device=dev)
         self._pack_stream = torch.cuda.Stream(device=dev)
@@ -195,11 +181,11 @@ class NerfTrainer:
         pack_into(self.coarse._desc, self.coarse._param_list(), self._pk[self.coarse])
         main.wait_event(self._ev3)
 
-    def _fwd(self, net, rays, P, out, acts, max_sms=0):
+    def _fwd(self, net, rays, P, out, acts):
         o, d, v, z = rays
         w, _, f = self._pk[net]
         call("ctx_mlp_fwd_ex", net._desc.p, ptr(w), ptr(f), 1, None, 0, ptr(o), ptr(d), ptr(v), ptr(z), z.shape[-1],
-             net.L_pts, net.L_dirs, P, ptr(out), ptr(acts), None, int(max_sms), stream_ptr(self.device))
+             net.L_pts, net.L_dirs, P, ptr(out), ptr(acts), None, 0, stream_ptr(self.device))
 
     def _dgrad(self, net, g_raw, acts, dacts, P, max_sms=0):
         _, wt, f = self._pk[net]
@@ -225,8 +211,6 @@ class NerfTrainer:
         Sf, Pc, Pf = S + Ni, pl.R * S, pl.R * (S + Ni)
         jit = self.perturb > 0.0
         main = torch.cuda.current_stream(dev)
-        early = self.overlap_backward and self.early_coarse
-        pl.fine_reduced = False
         call("ctx_step_tick", ptr(self._ctr), ptr(self._loss), stream_ptr(dev))
         self.bucket.zero_grad()
         ops.raygen(self.H, self.W, self.K, self.c2w, ray_idx=pl.idx, n_samples=S, near=self.near, far=self.far,
@@ -236,40 +220,18 @@ class NerfTrainer:
         self._timed("mlp_fwd_coarse", lambda: self._fwd(self.coarse, rays_c, Pc, pl.raw_c, pl.acts_c))
         # raw2outputs + img2mse(rgb0, target) + their backward in one pass; the weights feed sample_pdf
         self._comp_train(pl.raw_c, pl.z_c, pl.d, R, S, pl.target, pl.g_raw_c, pl.w_c, pl.rgb0)
-
-        def coarse_chain(dgrad_sms, wgrad_sms=0):
-            self._timed("mlp_dgrad_coarse",
-                        lambda: self._dgrad(self.coarse, pl.g_raw_c, pl.acts_c, pl.dacts_c, Pc, max_sms=dgrad_sms))
-            self._timed("mlp_wgrad_coarse",
-                        lambda: self._wgrad(self.coarse, pl.acts_c, pl.dacts_c, Pc, max_sms=wgrad_sms))
-
-        if early:
-            self._ev0.record(main)
-            self._side.wait_event(self._ev0)
-            with torch.cuda.stream(self._side):
-                coarse_chain(self.side_sms, self.side_sms)
-                self._ev1.record(self._side)
         ops.resample_merge(pl.z_c, pl.w_c, Ni, det=not jit, seed=self._seed0 + 1, seed_dev=self._ctr if jit else None,
                            out=(pl.zs, pl.z_f))
-        msm = self.main_sms if early else 0
-        self._timed("mlp_fwd_fine", lambda: self._fwd(self.fine, rays_f, Pf, pl.raw_f, pl.acts_f, max_sms=msm))
+        self._timed("mlp_fwd_fine", lambda: self._fwd(self.fine, rays_f, Pf, pl.raw_f, pl.acts_f))
         self._comp_train(pl.raw_f, pl.z_f, pl.d, R, Sf, pl.target, pl.g_raw_f, None, pl.rgb)
-        if self.sched_queue and self.overlap_backward and not early:
-            self._ev0.record(main)
-            self._side.wait_event(self._ev0)
-            self._dgrad(self.fine, pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf)
-            with torch.cuda.stream(self._side):
-                coarse_chain(0, 0)
-                self._ev1.record(self._side)
-            self._wgrad(self.fine, pl.acts_f, pl.dacts_f, Pf)
-            main.wait_event(self._ev1)
-            return
-        self._timed("mlp_dgrad_fine",
-                    lambda: self._dgrad(self.fine, pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf, max_sms=msm))
-        if early:
-            self._timed("mlp_wgrad_fine", lambda: self._wgrad(self.fine, pl.acts_f, pl.dacts_f, Pf))
-            main.wait_event(self._ev1)
-        elif self.overlap_backward:
+        self._timed("mlp_dgrad_fine", lambda: self._dgrad(self.fine, pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf))
+
+        def coarse_chain(dgrad_sms):
+            self._timed("mlp_dgrad_coarse",
+                        lambda: self._dgrad(self.coarse, pl.g_raw_c, pl.acts_c, pl.dacts_c, Pc, max_sms=dgrad_sms))
+            self._timed("mlp_wgrad_coarse", lambda: self._wgrad(self.coarse, pl.acts_c, pl.dacts_c, Pc))
+
+        if self.overlap_backward:
             self._ev0.record(main)
             self._side.wait_event(self._ev0)
             if self.timers is not None:
@@ -280,9 +242,6 @@ class NerfTrainer:
                 self._ev1.record(self._side)
             self._timed("mlp_wgrad_fine", lambda: self._wgrad(self.fine, pl.acts_f, pl.dacts_f, Pf,
                                                               max_sms=self.n_sms - self.side_sms))
-            if self.split_reduce and self.reduce_gradients:
-                self.comm.all_reduce(self.bucket.grad[self._n_coarse:])
-                pl.fine_reduced = True
             main.wait_event(self._ev1)
             if self.timers is not None:   # span of the concurrent group on the main stream
                 g1 = torch.cuda.Event(enable_timing=True)
@@ -328,12 +287,12 @@ class NerfTrainer:
             self._run(pl, optimizer_step)
         return self._loss
 
-    def _all_reduce(self, pl: _Plan):
-        """The exchange step after the join of the two backward chains (what the head has not already reduced)."""
+    def _all_reduce(self):
+        """The exchange step after the join of the two backward chains: the whole gradient bucket."""
         if not self.reduce_gradients:
             return
         if self.comm is not None:
-            self.comm.all_reduce(self.bucket.grad[:self._n_coarse] if pl.fine_reduced else self.bucket.grad)
+            self.comm.all_reduce(self.bucket.grad)
         else:
             self.bucket.all_reduce()
 
@@ -347,7 +306,7 @@ class NerfTrainer:
             # eager launch sequence (first step of a batch size: sets the kernels' attributes; timed passes)
             l0 = _lib.launch_count
             self._enqueue_head(pl)
-            self._all_reduce(pl)
+            self._all_reduce()
             if optimizer_step:
                 self._enqueue_tail()
             if graphable:
@@ -359,7 +318,7 @@ class NerfTrainer:
         _lib.launch_count += pl.kernels_per_step
         pl.graph.replay()
         if multi:
-            self._all_reduce(pl)
+            self._all_reduce()
             pl.graph_tail.replay()
 
     def _capture(self, pl: _Plan, multi: bool):
@@ -373,7 +332,7 @@ class NerfTrainer:
             with torch.cuda.graph(g, capture_error_mode="thread_local"):
                 self._enqueue_head(pl)
                 if not multi:
-                    self._all_reduce(pl)
+                    self._all_reduce()
                     self._enqueue_tail()
             tail = None
             if multi:

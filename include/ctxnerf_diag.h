@@ -1,8 +1,9 @@
 /* ctxnerf_diag.h -- diagnostics build of the library (libctxnerf_diag.so = the product sources compiled with
  * -DCTXNERF_DIAG + csrc/diag/tc_selftest.cu).  None of this is part of the drop-in boundary (include/ctxnerf.h):
- * tcgen05 / mbarrier micro-benchmarks, one-CTA GEMM self-tests that pin the descriptor conventions, and the hooks of
- * the profiling instantiation of the forward kernel (per-role cycle counters, deadlock reporter).  Used by tools/ and
- * by one GPU test; the product library exports none of these symbols.                                          */
+ * tcgen05 / mbarrier micro-benchmarks, one-CTA GEMM self-tests that pin the descriptor conventions, the hooks of
+ * the profiling instantiation of the forward kernel (per-role cycle counters, deadlock reporter) and the dgrad
+ * kernel's per-role cycle counters.  Used by tools/ and by one GPU test; the product library exports none of these
+ * symbols.                                                                                                      */
 #ifndef CTXNERF_DIAG_H
 #define CTXNERF_DIAG_H
 #include "ctxnerf.h"
@@ -16,6 +17,8 @@ int ctx_mlp_set_prof_buffer(void* device_u64);
 int ctx_mlp_set_debug(int flags);
 /* pinned host buffer the kernel's waiters report into before trapping when a barrier wait exceeds ~0.2 s */
 int ctx_mlp_set_hang_buffer(void* pinned_u64);
+/* dgrad kernel: 16 x uint64 per-role cycle counters per CTA (device pointer; NULL = off) */
+int ctx_dgrad_set_prof(void* device_u64);
 
 /* diagnostic: one-CTA tcgen05 GEMM C[128,N] = A * B^T (tests pin the descriptor
  * conventions with it); A,B bf16.  mode 0 K-major operands, 1 MN-major.          */

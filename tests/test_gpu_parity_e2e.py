@@ -324,7 +324,7 @@ def test_allreduced_gradients_of_two_ranks_equal_single_process_sum(cuda):
         pytest.skip("needs >= 2 GPUs")
     # both routes of the all-reduce: the library's NCCL binding (ctx_allreduce, a node of the step graph) and
     # torch.distributed between two graphs (CTXNERF_NCCL=0)
-    for k, (nccl, route) in enumerate((("1", "ctx_allreduce (NCCL"), ("0", "torch.distributed"))):     # (CTXNERF_SPLIT_REDUCE=1, the two-halves variant, is covered by tools/n2_allreduce_routes.sh)
+    for k, (nccl, route) in enumerate((("1", "ctx_allreduce (NCCL"), ("0", "torch.distributed"))):
         port = 29600 + (os.getpid() % 300) + k
         r = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
                             "--master-addr", "127.0.0.1", "--master-port", str(port),

@@ -7,7 +7,6 @@ print('$*', round(d['value']), round(d['ms_per_step'],4), round(d['e2e']['ms_per
 "; }
 for rep in 1 2; do
 run X=0
-run CTXNERF_SCHED=queue
 run CTXNERF_OVERLAP=0
 run CTXNERF_SIDE_SMS=52
 done

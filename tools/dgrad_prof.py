@@ -1,10 +1,10 @@
-"""Per-role cycle counters of the CTX_DG_PROF variant of mlp_dgrad_kernel (tools/build_variants.sh dgprof:"-DCTX_DG_PROF";
-run with CTXNERF_LIB=.../variants/libctxnerf_dgprof.so)."""
-import ctypes, os, sys
+"""Per-role cycle counters of mlp_dgrad_kernel, from the diagnostics build (libctxnerf_diag.so, include/ctxnerf_diag.h)."""
+import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path[:0] = [ROOT, os.path.join(ROOT, "contexture-nerf_b200")]
 import torch
-from ctxnerf import run_nerf_helpers as rh, _lib
+from ctxnerf import _lib as _l0; lib = _l0.use_diag_lib()   # diagnostics build (include/ctxnerf_diag.h)
+from ctxnerf import run_nerf_helpers as rh
 from ctxnerf.mlp import forward_raw
 from ctxnerf.mlp_bwd import mlp_dgrad
 dev = torch.device("cuda", 0)
@@ -16,8 +16,6 @@ z = torch.sort(torch.rand(R, S, device=dev) * 4 + 2, -1)[0]
 out, acts, P, packed = forward_raw(net, rays=(o, d, d, z), save_acts=True)
 g = torch.randn(P, 4, device=dev) / P
 prof = torch.zeros(148 * 16, dtype=torch.int64, device=dev)
-lib = _lib.lib()
-lib.ctx_dgrad_set_prof.argtypes = [ctypes.c_void_p]
 for _ in range(2):
     mlp_dgrad(net, packed, acts, P, g)
 torch.cuda.synchronize()

@@ -34,8 +34,7 @@ for b in batches:
 torch.cuda.synchronize()
 err = (reduced - ref).abs().max().item() / ref.abs().max().item()
 cos = torch.nn.functional.cosine_similarity(reduced, ref, dim=0).item()
-route = (f"ctx_allreduce (NCCL {tr.comm.version}{', fine half early' if tr.split_reduce else ''})"
-         if tr.comm is not None else "torch.distributed")
+route = f"ctx_allreduce (NCCL {tr.comm.version})" if tr.comm is not None else "torch.distributed"
 print(f"rank {rank}/{world}: all-reduced vs single-process sum: max rel err {err:.3e}, cosine {cos:.8f} [{route}]",
       flush=True)
 assert err < 1e-3 and cos > 0.999999

@@ -1,8 +1,8 @@
-# 2 GPUs: the three routes of the gradient all-reduce (correctness through tools/dist_check.py, then the bench line)
+# 2 GPUs: the two routes of the gradient all-reduce (correctness through tools/dist_check.py, then the bench line)
 TR="python -m torch.distributed.run --nnodes=1 --nproc-per-node 2 --master-addr 127.0.0.1"
 mkdir -p gpurun_out
 P=29520
-for v in "ctx_split:CTXNERF_NCCL=1 CTXNERF_SPLIT_REDUCE=1" "ctx_whole:CTXNERF_NCCL=1 CTXNERF_SPLIT_REDUCE=0" "torch:CTXNERF_NCCL=0"; do
+for v in "ctx:CTXNERF_NCCL=1" "torch:CTXNERF_NCCL=0"; do
   name=${v%%:*}; envs=${v#*:}
   env $envs timeout 300 $TR --master-port $P tools/dist_check.py > gpurun_out/dist2_$name.log 2>&1; echo "dist_check $name rc=$?"; P=$((P+1))
   if [ "$1" = "bench" ]; then

@@ -12,9 +12,6 @@ run CTXNERF_SIDE_SMS=36
 run CTXNERF_SIDE_SMS=52
 run CTXNERF_SIDE_SMS=60
 run CTXNERF_SIDE_SMS=28
-run CTXNERF_EARLY_COARSE=1 CTXNERF_SIDE_SMS=32
-run CTXNERF_EARLY_COARSE=1 CTXNERF_SIDE_SMS=44
-run CTXNERF_EARLY_COARSE=1 CTXNERF_SIDE_SMS=56
 run CTXNERF_OVERLAP=0
 run CTXNERF_GRAPH=0
 cat $out
