@@ -105,6 +105,48 @@ __device__ __forceinline__ void store_row(float* __restrict__ p, int64_t base, i
   }
 }
 
+// Density noise drawn inside the fused training pass (upstream raw2outputs: sigma + randn * raw_noise_std): sample s
+// of ray r gets std * n, n the standard normal philox_normal4 gives for (key, stream, row r, col s), with
+// key = seed + *seed_dev.  ctx_density_noise writes the same values as an [R,S] tensor.
+struct NoiseRng {
+  float std;
+  uint64_t seed;
+  const unsigned long long* seed_dev;   // nullable device counter added to seed (fresh numbers on every graph replay)
+  uint32_t stream;
+  __device__ __forceinline__ uint64_t key() const { return seed + (seed_dev ? *seed_dev : 0ull); }
+};
+
+// nz[k] = noise of samples s0 + k (k < K) of `ray`.  One Philox call serves a quad of samples; a lane whose K is a
+// multiple of 4 starts on a quad (s0 = multiple of K), a lane of 3 or 6 samples straddles quads and picks its samples
+// out of each quad it touches.
+template <int K>
+__device__ __forceinline__ void noise_row(const NoiseRng& g, uint64_t key, int64_t ray, int s0, float (&nz)[K + 1]) {
+  const uint32_t q0 = (uint32_t)s0 >> 2;
+  if constexpr ((K & 3) == 0) {
+#pragma unroll
+    for (int q = 0; q < K / 4; ++q) {
+      const float4 n = philox_normal4(key, g.stream, (uint64_t)ray, q0 + q);
+      nz[4 * q + 0] = __fmul_rn(g.std, n.x); nz[4 * q + 1] = __fmul_rn(g.std, n.y);
+      nz[4 * q + 2] = __fmul_rn(g.std, n.z); nz[4 * q + 3] = __fmul_rn(g.std, n.w);
+    }
+  } else {
+    const int off = s0 & 3;
+    constexpr int NQ = (K + 6) / 4;              // most quads K consecutive samples can touch
+#pragma unroll
+    for (int j = 0; j < NQ; ++j) {
+      if (4 * j < off + K) {
+        const float4 n = philox_normal4(key, g.stream, (uint64_t)ray, q0 + j);
+        const float v[4] = {n.x, n.y, n.z, n.w};
+#pragma unroll
+        for (int k = 0; k < K; ++k)
+#pragma unroll
+          for (int e = 0; e < 4; ++e)
+            if (4 * j + e == off + k) nz[k] = __fmul_rn(g.std, v[e]);
+      }
+    }
+  }
+}
+
 // G lanes share a ray (32 / G rays per warp): short rays use 8- or 16-lane groups so that the scan and the five
 // reductions, the part of the work that does not shrink with S, are paid once per 4 or 2 rays.
 template <int K, int G>
@@ -197,7 +239,8 @@ composite_fwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
 // gradient g_rgb = 2 (rgb_map - target) * loss_scale are formed in place -- one pass over raw replaces
 // composite_fwd + mse + composite_bwd.  It writes g_raw, optionally weights (the coarse pass feeds sample_pdf) and
 // rgb_map; the loss itself is summed from rgb_map by loss_sum_kernel, in a fixed order.
-template <int K, int G, bool TRAIN>
+// RNG = true (TRAIN only): the density noise comes from `rng` instead of the `noise` rows.
+template <int K, int G, bool TRAIN, bool RNG>
 __global__ void __launch_bounds__(kCompWarps * 32, K <= 4 ? 4 : (K <= 8 ? 2 : 1))
 composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z,
                      const float* __restrict__ rays_d, const float* __restrict__ noise,
@@ -206,12 +249,14 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
                      const float* __restrict__ g_acc, const float* __restrict__ g_weights,
                      const float* __restrict__ g_depth, float4* __restrict__ g_raw,
                      const float* __restrict__ target, float loss_scale, float* __restrict__ loss,
-                     float* __restrict__ weights_out, float* __restrict__ rgb_out) {
+                     float* __restrict__ weights_out, float* __restrict__ rgb_out, NoiseRng rng) {
   constexpr int RPW = 32 / G;
   const int lane = threadIdx.x & (G - 1), sub = (threadIdx.x & 31) / G;
   const int64_t warp0 = (int64_t)blockIdx.x * kCompWarps + (threadIdx.x >> 5);
   const int64_t nwarps = (int64_t)gridDim.x * kCompWarps;
   const int s0 = lane * K;
+  uint64_t key = 0;
+  if constexpr (RNG) key = rng.key();
   for (int64_t rb = warp0 * RPW; rb < R; rb += nwarps * RPW) {
     const bool live = rb + sub < R;
     const int64_t ray = live ? rb + sub : R - 1;
@@ -225,7 +270,8 @@ composite_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z
     for (int k = 0; k < K; ++k)
       rw[k] = (s0 + k < S) ? __ldg(raw + base + s0 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
     load_row<K>(z, base, s0, S, vec, zl);
-    if (noise != nullptr) load_row<K>(noise, base, s0, S, vec, nz);
+    if constexpr (RNG) noise_row<K>(rng, key, ray, s0, nz);
+    else if (noise != nullptr) load_row<K>(noise, base, s0, S, vec, nz);
     else {
 #pragma unroll
       for (int k = 0; k < K; ++k) nz[k] = 0.f;
@@ -372,20 +418,27 @@ __device__ __forceinline__ int dev_vec(int S, const void* a, const void* b, cons
   return ((S & 3) == 0 && (bits & 15) == 0) ? 4 : 1;
 }
 
-template <int K>
+template <int K, bool RNG = false>
 __device__ __forceinline__ void chunk_load(const float4* __restrict__ raw, const float* __restrict__ z,
                                            const float* __restrict__ noise, int64_t base, int c0, int lane, int S,
                                            int vec, float dnorm, float4 (&rw)[K], float (&zl)[K + 1], float (&sig)[K],
-                                           float (&dist)[K]) {
+                                           float (&dist)[K], const NoiseRng* rng = nullptr, uint64_t key = 0,
+                                           int64_t ray = 0) {
   const int s0 = c0 + lane * K;
 #pragma unroll
   for (int k = 0; k < K; ++k)
     rw[k] = (s0 + k < S) ? __ldg(raw + base + s0 + k) : make_float4(0.f, 0.f, 0.f, 0.f);
   load_row<K>(z, base, s0, S, vec, zl);                        // 16-byte pieces when the rows allow it
   float nz[K + 1];
-  if (noise != nullptr) load_row<K>(noise, base, s0, S, vec, nz);
+  if constexpr (RNG) {
+    noise_row<K>(*rng, key, ray, s0, nz);
 #pragma unroll
-  for (int k = 0; k < K; ++k) sig[k] = rw[k].w + (noise != nullptr ? nz[k] : 0.f);
+    for (int k = 0; k < K; ++k) sig[k] = rw[k].w + nz[k];
+  } else {
+    if (noise != nullptr) load_row<K>(noise, base, s0, S, vec, nz);
+#pragma unroll
+    for (int k = 0; k < K; ++k) sig[k] = rw[k].w + (noise != nullptr ? nz[k] : 0.f);
+  }
   zl[K] = (s0 + K < S) ? __ldg(z + base + s0 + K) : 0.f;     // first depth of the next lane / next chunk
 #pragma unroll
   for (int k = 0; k < K; ++k) {
@@ -454,7 +507,7 @@ composite_chunked_fwd_kernel(const float4* __restrict__ raw, const float* __rest
 
 // backward / fused training form over chunks: pass 1 walks forward (entry transmittance of every chunk, ray totals),
 // pass 2 walks the chunks in reverse with the incoming value of U (see composite_bwd_kernel for the recurrence).
-template <int K, bool TRAIN>
+template <int K, bool TRAIN, bool RNG>
 __global__ void __launch_bounds__(kCompWarps * 32)
 composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __restrict__ z,
                              const float* __restrict__ rays_d, const float* __restrict__ noise, int64_t R, int S,
@@ -462,13 +515,15 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
                              const float* __restrict__ g_acc, const float* __restrict__ g_weights,
                              const float* __restrict__ g_depth, float4* __restrict__ g_raw,
                              const float* __restrict__ target, float loss_scale, float* __restrict__ loss,
-                             float* __restrict__ weights_out, float* __restrict__ rgb_out) {
+                             float* __restrict__ weights_out, float* __restrict__ rgb_out, NoiseRng rng) {
   __shared__ float s_carry[kCompWarps][kCompMaxChunks];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
   const int64_t warp0 = (int64_t)blockIdx.x * kCompWarps + wib;
   const int64_t nwarps = (int64_t)gridDim.x * kCompWarps;
   const int n_chunks = (S + 32 * K - 1) / (32 * K);
   const int vec = dev_vec(S, z, noise, TRAIN ? (const void*)weights_out : (const void*)g_weights);
+  uint64_t key = 0;
+  if constexpr (RNG) key = rng.key();
   for (int64_t ray = warp0; ray < R; ray += nwarps) {
     const float dx = rays_d[ray * 3 + 0], dy = rays_d[ray * 3 + 1], dz = rays_d[ray * 3 + 2];
     const float dnorm = sqrtf(dx * dx + dy * dy + dz * dz);
@@ -479,7 +534,7 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
       const int c0 = ci * 32 * K;
       float4 rw[K];
       float zl[K + 1], sig[K], dist[K];
-      chunk_load<K>(raw, z, noise, base, c0, lane, S, vec, dnorm, rw, zl, sig, dist);
+      chunk_load<K, RNG>(raw, z, noise, base, c0, lane, S, vec, dnorm, rw, zl, sig, dist, &rng, key, ray);
       if (lane == 0) s_carry[wib][ci] = carry;
       float al[K], pref[K];
       float run = 1.0f;
@@ -544,7 +599,7 @@ composite_chunked_bwd_kernel(const float4* __restrict__ raw, const float* __rest
       const int c0 = ci * 32 * K;
       float4 rw[K];
       float zl[K + 1], sig[K], dist[K];
-      chunk_load<K>(raw, z, noise, base, c0, lane, S, vec, dnorm, rw, zl, sig, dist);
+      chunk_load<K, RNG>(raw, z, noise, base, c0, lane, S, vec, dnorm, rw, zl, sig, dist, &rng, key, ray);
       const float cin = s_carry[wib][ci];
       float ex[K], pref[K], Gs[K];
       float run = 1.0f;
@@ -642,15 +697,15 @@ static inline int comp_grid(int64_t R, int S) {
   else if (S <= 384) KERNEL<12, 32><<<grid, block, 0, st>>>(__VA_ARGS__);                  \
   else KERNEL<16, 32><<<grid, block, 0, st>>>(__VA_ARGS__);
 
-#define CTX_COMP_DISPATCH_BWD(TRAIN, ...)                                                                   \
-  if (S <= 32) ctx::composite_bwd_kernel<4, 8, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);                    \
-  else if (S <= 64) ctx::composite_bwd_kernel<4, 16, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);              \
-  else if (S <= 96) ctx::composite_bwd_kernel<3, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);              \
-  else if (S <= 128) ctx::composite_bwd_kernel<4, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);             \
-  else if (S <= 192) ctx::composite_bwd_kernel<6, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);             \
-  else if (S <= 256) ctx::composite_bwd_kernel<8, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);             \
-  else if (S <= 384) ctx::composite_bwd_kernel<12, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);            \
-  else ctx::composite_bwd_kernel<16, 32, TRAIN><<<grid, block, 0, st>>>(__VA_ARGS__);
+#define CTX_COMP_DISPATCH_BWD(TRAIN, RNG, ...)                                                                   \
+  if (S <= 32) ctx::composite_bwd_kernel<4, 8, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);                    \
+  else if (S <= 64) ctx::composite_bwd_kernel<4, 16, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);              \
+  else if (S <= 96) ctx::composite_bwd_kernel<3, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);              \
+  else if (S <= 128) ctx::composite_bwd_kernel<4, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);             \
+  else if (S <= 192) ctx::composite_bwd_kernel<6, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);             \
+  else if (S <= 256) ctx::composite_bwd_kernel<8, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);             \
+  else if (S <= 384) ctx::composite_bwd_kernel<12, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);            \
+  else ctx::composite_bwd_kernel<16, 32, TRAIN, RNG><<<grid, block, 0, st>>>(__VA_ARGS__);
 
 extern "C" int ctx_composite_fwd(const float* raw, const float* z_vals, const float* rays_d,
                                  const float* noise, int64_t R, int S, int white_bkgd,
@@ -689,14 +744,15 @@ extern "C" int ctx_composite_bwd(const float* raw, const float* z_vals, const fl
   cudaStream_t st = (cudaStream_t)stream;
   const int grid = ctx::comp_grid(R, S), block = ctx::kCompWarps * 32;
   if (S > ctx::comp_single_pass_max()) {
-    ctx::composite_chunked_bwd_kernel<8, false><<<grid, block, 0, st>>>(
+    ctx::composite_chunked_bwd_kernel<8, false, false><<<grid, block, 0, st>>>(
         (const float4*)raw, z_vals, rays_d, noise, R, S, white_bkgd, g_rgb, g_disp, g_acc, g_weights, g_depth,
-        (float4*)g_raw, nullptr, 0.f, nullptr, nullptr, nullptr);
+        (float4*)g_raw, nullptr, 0.f, nullptr, nullptr, nullptr, ctx::NoiseRng{});
     CTX_RETURN_LAST();
   }
   const int vec = ctx::comp_vec(S, {z_vals, noise, g_weights});
-  CTX_COMP_DISPATCH_BWD(false, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, g_rgb, g_disp,
-                        g_acc, g_weights, g_depth, (float4*)g_raw, nullptr, 0.f, nullptr, nullptr, nullptr)
+  CTX_COMP_DISPATCH_BWD(false, false, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, g_rgb,
+                        g_disp, g_acc, g_weights, g_depth, (float4*)g_raw, nullptr, 0.f, nullptr, nullptr, nullptr,
+                        ctx::NoiseRng{})
   CTX_RETURN_LAST();
 }
 
@@ -723,6 +779,47 @@ __global__ void __launch_bounds__(1024) loss_sum_kernel(const float* __restrict_
 }
 }  // namespace ctx
 
+namespace ctx {
+// the launches behind ctx_composite_train (RNG = false: the `noise` rows, if any) and ctx_composite_train_noise
+// (RNG = true: noise drawn in-kernel from `rng`)
+template <bool RNG>
+static int composite_train_launch(const float* raw, const float* z_vals, const float* rays_d, const float* noise,
+                                  int64_t R, int S, int white_bkgd, const float* target, float loss_scale, float* loss,
+                                  float* g_raw, float* weights, float* rgb_map, NoiseRng rng, cudaStream_t st) {
+  const int grid = comp_grid(R, S), block = kCompWarps * 32;
+  if (S > comp_single_pass_max()) {
+    composite_chunked_bwd_kernel<8, true, RNG><<<grid, block, 0, st>>>(
+        (const float4*)raw, z_vals, rays_d, noise, R, S, white_bkgd, nullptr, nullptr, nullptr, nullptr, nullptr,
+        (float4*)g_raw, target, loss_scale, nullptr, weights, rgb_map, rng);
+  } else {
+    const int vec = comp_vec(S, {z_vals, noise, weights});
+    CTX_COMP_DISPATCH_BWD(true, RNG, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, nullptr,
+                          nullptr, nullptr, nullptr, nullptr, (float4*)g_raw, target, loss_scale, nullptr, weights,
+                          rgb_map, rng)
+  }
+  loss_sum_kernel<<<1, 1024, 0, st>>>(rgb_map, target, R, loss_scale, loss);
+  CTX_RETURN_LAST();
+}
+
+// [R,S] rows of the in-kernel density noise: one thread per quad of samples, the Philox call the fused pass makes
+__global__ void density_noise_kernel(float* __restrict__ out, int64_t R, int S, NoiseRng g) {
+  const uint64_t key = g.key();
+  const int nq = (S + 3) >> 2;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < R * nq; i += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t r = i / nq;
+    const int q = (int)(i - r * nq);
+    const float4 n = philox_normal4(key, g.stream, (uint64_t)r, (uint32_t)q);
+    const float v[4] = {n.x, n.y, n.z, n.w};
+#pragma unroll
+    for (int e = 0; e < 4; ++e)
+      if (4 * q + e < S) out[r * S + 4 * q + e] = __fmul_rn(g.std, v[e]);
+  }
+}
+
+// streams 0 and 1 of the step's key are the stratified jitter and the sample_pdf uniforms
+static inline bool noise_args_ok(float noise_std, int stream_id) { return noise_std >= 0.f && stream_id >= 2; }
+}  // namespace ctx
+
 // Fused training form of raw2outputs: forward + img2mse(rgb_map, target) + backward in one pass (see the kernel),
 // then the loss from rgb_map (loss_sum_kernel).  loss_scale = 1 / (3 R) for the mean over the rgb image; loss[0] is
 // ADDED to (zero it once per step: the coarse and the fine pass accumulate into the same scalar).  weights is an
@@ -735,17 +832,39 @@ extern "C" int ctx_composite_train(const float* raw, const float* z_vals, const 
   if (!raw || !z_vals || !rays_d || !target || !loss || !g_raw || !rgb_map) return CTX_ERR_BAD_ARG;
   if (reinterpret_cast<uintptr_t>(raw) % 16 != 0 || reinterpret_cast<uintptr_t>(g_raw) % 16 != 0)
     return CTX_ERR_BAD_ARG;
+  return ctx::composite_train_launch<false>(raw, z_vals, rays_d, noise, R, S, white_bkgd, target, loss_scale, loss,
+                                            g_raw, weights, rgb_map, ctx::NoiseRng{}, (cudaStream_t)stream);
+}
+
+// ctx_composite_train with the density noise noise_std * n drawn inside the kernel (the values ctx_density_noise
+// writes), so that a captured training step needs no noise tensor made before each replay.  noise_std == 0 runs
+// exactly the launches of ctx_composite_train without noise.
+extern "C" int ctx_composite_train_noise(const float* raw, const float* z_vals, const float* rays_d, int64_t R, int S,
+                                         int white_bkgd, const float* target, float loss_scale, float* loss,
+                                         float* g_raw, float* weights, float* rgb_map, float noise_std, uint64_t seed,
+                                         const uint64_t* seed_dev, int stream_id, void* stream) {
+  if (R < 0 || S < 1 || S > 256 * ctx::kCompMaxChunks || !ctx::noise_args_ok(noise_std, stream_id))
+    return CTX_ERR_BAD_ARG;
+  if (!raw || !z_vals || !rays_d || !target || !loss || !g_raw || !rgb_map) return CTX_ERR_BAD_ARG;
+  if (reinterpret_cast<uintptr_t>(raw) % 16 != 0 || reinterpret_cast<uintptr_t>(g_raw) % 16 != 0)
+    return CTX_ERR_BAD_ARG;
+  if (R == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
-  const int grid = ctx::comp_grid(R, S), block = ctx::kCompWarps * 32;
-  if (S > ctx::comp_single_pass_max()) {
-    ctx::composite_chunked_bwd_kernel<8, true><<<grid, block, 0, st>>>(
-        (const float4*)raw, z_vals, rays_d, noise, R, S, white_bkgd, nullptr, nullptr, nullptr, nullptr, nullptr,
-        (float4*)g_raw, target, loss_scale, nullptr, weights, rgb_map);
-  } else {
-    const int vec = ctx::comp_vec(S, {z_vals, noise, weights});
-    CTX_COMP_DISPATCH_BWD(true, (const float4*)raw, z_vals, rays_d, noise, R, S, vec, white_bkgd, nullptr, nullptr,
-                          nullptr, nullptr, nullptr, (float4*)g_raw, target, loss_scale, nullptr, weights, rgb_map)
-  }
-  ctx::loss_sum_kernel<<<1, 1024, 0, st>>>(rgb_map, target, R, loss_scale, loss);
+  if (noise_std == 0.f)
+    return ctx::composite_train_launch<false>(raw, z_vals, rays_d, nullptr, R, S, white_bkgd, target, loss_scale,
+                                              loss, g_raw, weights, rgb_map, ctx::NoiseRng{}, st);
+  const ctx::NoiseRng rng{noise_std, seed, reinterpret_cast<const unsigned long long*>(seed_dev), (uint32_t)stream_id};
+  return ctx::composite_train_launch<true>(raw, z_vals, rays_d, nullptr, R, S, white_bkgd, target, loss_scale, loss,
+                                           g_raw, weights, rgb_map, rng, st);
+}
+
+extern "C" int ctx_density_noise(float* noise, int64_t R, int S, float noise_std, uint64_t seed,
+                                 const uint64_t* seed_dev, int stream_id, void* stream) {
+  if (R < 0 || S < 1 || !noise || !ctx::noise_args_ok(noise_std, stream_id)) return CTX_ERR_BAD_ARG;
+  if (R == 0) return 0;
+  int64_t blocks = ctx::ceil_div(R * ((S + 3) / 4), 256);
+  if (blocks > ctx::num_sms() * 8) blocks = ctx::num_sms() * 8;
+  const ctx::NoiseRng rng{noise_std, seed, reinterpret_cast<const unsigned long long*>(seed_dev), (uint32_t)stream_id};
+  ctx::density_noise_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(noise, R, S, rng);
   CTX_RETURN_LAST();
 }

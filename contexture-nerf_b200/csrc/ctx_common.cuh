@@ -86,6 +86,22 @@ __device__ __forceinline__ float philox_uniform(uint64_t seed, uint64_t stream, 
   return u01(sel == 0 ? r.x : sel == 1 ? r.y : sel == 2 ? r.z : r.w);
 }
 
+// four standard normals for (stream, row, cols 4q .. 4q+3): the Philox call of philox_uniform's layout, then
+// Box-Muller on (x, y) and (z, w), cos then sin.  The radius uniform lies in (0, 1] so that log never sees 0 (|n| is
+// at most sqrt(48 ln 2) = 5.77).  Explicitly rounded products: callers that inline this keep the same bits whatever
+// they do with the result.
+__device__ __forceinline__ float4 philox_normal4(uint64_t seed, uint64_t stream, uint64_t row, uint32_t quad) {
+  Philox ph(seed);
+  const uint4 r = ph(row, (stream << 32) | (uint64_t)quad);
+  const float ua = (float)((r.x >> 8) + 1u) * (1.0f / 16777216.0f), ta = u01(r.y);
+  const float ub = (float)((r.z >> 8) + 1u) * (1.0f / 16777216.0f), tb = u01(r.w);
+  const float ra = sqrtf(__fmul_rn(-2.0f, logf(ua))), rb = sqrtf(__fmul_rn(-2.0f, logf(ub)));
+  float sa, ca, sb, cb;
+  sincospif(__fmul_rn(2.0f, ta), &sa, &ca);
+  sincospif(__fmul_rn(2.0f, tb), &sb, &cb);
+  return make_float4(__fmul_rn(ra, ca), __fmul_rn(ra, sa), __fmul_rn(rb, cb), __fmul_rn(rb, sb));
+}
+
 // cudaFuncSetAttribute is per device: remember which devices a launcher has already prepared (one process may drive
 // several GPUs even though the training path uses one process per GPU)
 struct DeviceOnce {

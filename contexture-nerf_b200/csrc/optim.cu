@@ -32,11 +32,17 @@ __global__ void step_tick_kernel(unsigned long long* __restrict__ ctr, float* __
   }
 }
 
-// Adam with the step count read from the device counter (bias corrections formed per thread: two powf)
+// Adam with the step count read from the device counter (bias corrections formed per thread: two powf).
+// DECAY: update t uses lr * 0.1^(max(t-2, 0) / decay_steps), the rate upstream's loop has set when its t-th
+// optimizer.step() runs (it sets lrate * 0.1^(global_step / decay_steps) after each step, then counts global_step
+// up from 0).
+template <bool DECAY>
 __global__ void adam_dev_kernel(float* __restrict__ p, const float* __restrict__ g, float* __restrict__ m,
                                 float* __restrict__ v, int64_t n, float lr, float b1, float b2, float eps,
-                                const unsigned long long* __restrict__ ctr, float wd, float grad_scale) {
+                                const unsigned long long* __restrict__ ctr, float wd, float grad_scale,
+                                float decay_steps) {
   const float step = (float)ctr[1];
+  if constexpr (DECAY) lr *= powf(0.1f, fmaxf(step - 2.f, 0.f) / decay_steps);
   const float bc1 = 1.f - powf(b1, step);
   const float bc2_sqrt = sqrtf(1.f - powf(b2, step));
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
@@ -144,9 +150,23 @@ extern "C" int ctx_adam_step_dev(float* params, const float* grads, float* exp_a
   if (n == 0) return 0;
   int64_t blocks = ctx::ceil_div(n, 256);
   if (blocks > ctx::num_sms() * 8) blocks = ctx::num_sms() * 8;
-  ctx::adam_dev_kernel<<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(params, grads, exp_avg, exp_avg_sq, n, lr, beta1,
-                                                                      beta2, eps, (const unsigned long long*)counters,
-                                                                      weight_decay, grad_scale);
+  ctx::adam_dev_kernel<false><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+      params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, (const unsigned long long*)counters, weight_decay,
+      grad_scale, 0.f);
+  CTX_RETURN_LAST();
+}
+
+extern "C" int ctx_adam_step_dev_decay(float* params, const float* grads, float* exp_avg, float* exp_avg_sq,
+                                       int64_t n, float lr, float beta1, float beta2, float eps, const void* counters,
+                                       float weight_decay, float grad_scale, float decay_steps, void* stream) {
+  if (n < 0 || !params || !grads || !exp_avg || !exp_avg_sq || !counters || !(decay_steps > 0.f))
+    return CTX_ERR_BAD_ARG;
+  if (n == 0) return 0;
+  int64_t blocks = ctx::ceil_div(n, 256);
+  if (blocks > ctx::num_sms() * 8) blocks = ctx::num_sms() * 8;
+  ctx::adam_dev_kernel<true><<<(int)blocks, 256, 0, (cudaStream_t)stream>>>(
+      params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, (const unsigned long long*)counters, weight_decay,
+      grad_scale, decay_steps);
   CTX_RETURN_LAST();
 }
 

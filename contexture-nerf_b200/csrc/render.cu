@@ -13,7 +13,9 @@
 // sizeof(CtxRenderArgs) as this library was compiled: lets a binding check its own struct layout
 extern "C" int ctx_render_args_bytes(void) { return (int)sizeof(CtxRenderArgs); }
 
-extern "C" int ctx_render_rays(const CtxRenderArgs* a, void* stream) {
+// use_ndc: the raygen launch warps the rays to NDC (ndc_rays(H, W, ndc_focal, ndc_near, ...)) after taking the view
+// directions, as upstream render() does for forward-facing scenes; near / far are then NDC depths.
+static int render_rays(const CtxRenderArgs* a, int use_ndc, float ndc_focal, float ndc_near, void* stream) {
   if (!a || a->n_rays < 0 || a->n_samples < 2 || a->n_importance < 0) return CTX_ERR_BAD_ARG;
   if (a->n_rays == 0) return 0;
   const int S = a->n_samples, Ni = a->n_importance, Sf = S + Ni;
@@ -29,8 +31,8 @@ extern "C" int ctx_render_rays(const CtxRenderArgs* a, void* stream) {
   const CtxNet& fine = a->fine.desc ? a->fine : a->coarse;        // network_fine or network_fn
   if (!fine.wpacked || !fine.fparams) return CTX_ERR_BAD_ARG;
 
-  int rc = ctx_raygen_fwd(a->H, a->W, a->fx, a->fy, a->cx, a->cy, a->c2w, a->c2w_ld, a->ray_idx, R, 0, 0.f, 0.f, S,
-                          a->near, a->far, a->lindisp, a->perturb, nullptr, a->seed, a->seed_dev,
+  int rc = ctx_raygen_fwd(a->H, a->W, a->fx, a->fy, a->cx, a->cy, a->c2w, a->c2w_ld, a->ray_idx, R, use_ndc,
+                          ndc_focal, ndc_near, S, a->near, a->far, a->lindisp, a->perturb, nullptr, a->seed, a->seed_dev,
                           a->sphere != nullptr, a->sphere, a->rays_o, a->rays_d, a->viewdirs, a->z_coarse, nullptr,
                           stream);
   if (rc) return rc;
@@ -53,4 +55,12 @@ extern "C" int ctx_render_rays(const CtxRenderArgs* a, void* stream) {
   if (rc) return rc;
   return ctx_composite_fwd(a->raw_fine, a->z_fine, a->rays_d, nullptr, R, Sf, a->white_bkgd, a->rgb_map, a->disp_map,
                            a->acc_map, a->weights_fine, a->depth_map, stream);
+}
+
+extern "C" int ctx_render_rays(const CtxRenderArgs* a, void* stream) { return render_rays(a, 0, 0.f, 0.f, stream); }
+
+extern "C" int ctx_render_rays_ndc(const CtxRenderArgs* a, float ndc_focal, float ndc_near, void* stream) {
+  // the bounding-sphere interval is metric: it has no meaning for NDC rays
+  if (!a || !(ndc_focal > 0.f) || !(ndc_near > 0.f) || a->sphere) return CTX_ERR_BAD_ARG;
+  return render_rays(a, 1, ndc_focal, ndc_near, stream);
 }

@@ -68,9 +68,25 @@ class _Plan:
 
 
 class NerfTrainer:
+    """Upstream nerf-pytorch's training step for one camera.  The defaults are its Blender recipe; its forward-facing
+    (LLFF) recipe is ``ndc=True, near=0, far=1, raw_noise_std=1.0, lrate_decay=250, white_bkgd=False``:
+
+    * ``ndc``: rays are warped by ``ndc_rays(H, W, K[0][0], 1., ...)`` after the view directions are taken, so
+      near / far are NDC depths.  Training, ``render`` and ``render_view`` all use the warped rays.
+    * ``raw_noise_std``: the training step adds ``raw_noise_std * randn`` to every density, drawn inside the fused
+      compositing kernels (Philox key ``seed0 + counter``, stream 2 coarse, 3 fine): fresh on every step, reproducible
+      under ``torch.manual_seed``.  Renders stay noise-free, as upstream's ``render_kwargs_test``.
+    * ``lrate_decay`` (thousands of steps): Adam's update ``t`` uses
+      ``lr * 0.1 ** (max(t - 2, 0) / (lrate_decay * 1000))``, the rate upstream's loop sets; 0 keeps ``lr`` constant.
+    """
+
     def __init__(self, H, W, K, c2w, near=2.0, far=6.0, N_samples=64, N_importance=128, perturb=1.0,
                  white_bkgd=True, lindisp=False, lr=5e-4, betas=(0.9, 0.999), eps=1e-8, device=None, seed=0,
-                 multires=10, multires_views=4):
+                 multires=10, multires_views=4, ndc=False, raw_noise_std=0.0, lrate_decay=0):
+        if not raw_noise_std >= 0.0:
+            raise CtxNerfError("NerfTrainer: raw_noise_std must be >= 0")
+        if not lrate_decay >= 0:
+            raise CtxNerfError("NerfTrainer: lrate_decay must be >= 0 (thousands of steps; 0 = constant rate)")
         self.device = torch.device(device if device is not None else ("cuda", torch.cuda.current_device()))
         dev = self.device
         self.H, self.W, self.K = H, W, K
@@ -79,6 +95,7 @@ class NerfTrainer:
         self.N_samples, self.N_importance = int(N_samples), int(N_importance)
         self.perturb, self.white_bkgd, self.lindisp = float(perturb), bool(white_bkgd), bool(lindisp)
         self.lr, self.betas, self.eps = lr, betas, eps
+        self.ndc, self.raw_noise_std, self.lrate_decay = bool(ndc), float(raw_noise_std), lrate_decay
         # identical initial weights on every rank: construct under a fixed seed
         st = torch.random.get_rng_state()
         torch.manual_seed(seed)
@@ -106,7 +123,7 @@ class NerfTrainer:
         # device-side step state: [0] Philox seed offset, [1] Adam step count (ctx_step_tick advances both)
         self._ctr = torch.zeros(2, device=dev, dtype=torch.int64)
         # the Philox base seed comes from torch's generator: torch.manual_seed makes a training run reproducible
-        self._seed0 = ops.new_seed() if self.perturb > 0.0 else 0
+        self._seed0 = ops.new_seed() if self.perturb > 0.0 or self.raw_noise_std > 0.0 else 0
         # bf16 weight streams of both networks: trainer-owned static buffers, re-packed after every Adam update
         self._pk = {}
         for net in (self.coarse, self.fine):
@@ -200,7 +217,12 @@ class NerfTrainer:
         call("ctx_mlp_wgrad_ex", net._desc.p, ptr(acts), ptr(dacts), P, ctypes.cast(garr, ctypes.c_void_p), len(sinks),
              ctypes.cast(parr, ctypes.c_void_p), ptr(self._scratch[net]), int(max_sms), stream_ptr(self.device))
 
-    def _comp_train(self, raw, z, d, R, S, target, g_raw, weights, rgb):
+    def _comp_train(self, raw, z, d, R, S, target, g_raw, weights, rgb, noise_stream):
+        if self.raw_noise_std > 0.0:     # the raygen key (seed0 + counter), its own Philox stream per pass
+            call("ctx_composite_train_noise", ptr(raw), ptr(z), ptr(d), R, S, int(self.white_bkgd), ptr(target),
+                 1.0 / (3.0 * R), ptr(self._loss), ptr(g_raw), ptr(weights), ptr(rgb), self.raw_noise_std,
+                 self._seed0, ptr(self._ctr), noise_stream, stream_ptr(self.device))
+            return
         call("ctx_composite_train", ptr(raw), ptr(z), ptr(d), None, R, S, int(self.white_bkgd), ptr(target),
              1.0 / (3.0 * R), ptr(self._loss), ptr(g_raw), ptr(weights), ptr(rgb), stream_ptr(self.device))
 
@@ -215,15 +237,15 @@ class NerfTrainer:
         self.bucket.zero_grad()
         ops.raygen(self.H, self.W, self.K, self.c2w, ray_idx=pl.idx, n_samples=S, near=self.near, far=self.far,
                    lindisp=self.lindisp, perturb=jit, seed=self._seed0, seed_dev=self._ctr if jit else None,
-                   want_viewdirs=True, out=(pl.o, pl.d, pl.v, pl.z_c))
+                   ndc=self._ndc_args(self.K), want_viewdirs=True, out=(pl.o, pl.d, pl.v, pl.z_c))
         rays_c, rays_f = (pl.o, pl.d, pl.v, pl.z_c), (pl.o, pl.d, pl.v, pl.z_f)
         self._timed("mlp_fwd_coarse", lambda: self._fwd(self.coarse, rays_c, Pc, pl.raw_c, pl.acts_c))
         # raw2outputs + img2mse(rgb0, target) + their backward in one pass; the weights feed sample_pdf
-        self._comp_train(pl.raw_c, pl.z_c, pl.d, R, S, pl.target, pl.g_raw_c, pl.w_c, pl.rgb0)
+        self._comp_train(pl.raw_c, pl.z_c, pl.d, R, S, pl.target, pl.g_raw_c, pl.w_c, pl.rgb0, 2)
         ops.resample_merge(pl.z_c, pl.w_c, Ni, det=not jit, seed=self._seed0 + 1, seed_dev=self._ctr if jit else None,
                            out=(pl.zs, pl.z_f))
         self._timed("mlp_fwd_fine", lambda: self._fwd(self.fine, rays_f, Pf, pl.raw_f, pl.acts_f))
-        self._comp_train(pl.raw_f, pl.z_f, pl.d, R, Sf, pl.target, pl.g_raw_f, None, pl.rgb)
+        self._comp_train(pl.raw_f, pl.z_f, pl.d, R, Sf, pl.target, pl.g_raw_f, None, pl.rgb, 3)
         self._timed("mlp_dgrad_fine", lambda: self._dgrad(self.fine, pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf))
 
         def coarse_chain(dgrad_sms):
@@ -253,9 +275,13 @@ class NerfTrainer:
 
     def _enqueue_tail(self):
         dev = self.device
-        call("ctx_adam_step_dev", ptr(self.bucket.flat), ptr(self.bucket.grad), ptr(self.exp_avg),
-             ptr(self.exp_avg_sq), self.bucket.numel, self.lr, self.betas[0], self.betas[1], self.eps, ptr(self._ctr),
-             0.0, 1.0 / self.world_size, stream_ptr(dev))
+        args = (ptr(self.bucket.flat), ptr(self.bucket.grad), ptr(self.exp_avg), ptr(self.exp_avg_sq),
+                self.bucket.numel, self.lr, self.betas[0], self.betas[1], self.eps, ptr(self._ctr), 0.0,
+                1.0 / self.world_size)
+        if self.lrate_decay > 0:
+            call("ctx_adam_step_dev_decay", *args, float(self.lrate_decay) * 1000.0, stream_ptr(dev))
+        else:
+            call("ctx_adam_step_dev", *args, stream_ptr(dev))
         self._repack()
 
     def _plan(self, R: int) -> _Plan:
@@ -263,6 +289,17 @@ class NerfTrainer:
         if pl is None:
             pl = self._plans[R] = _Plan(self, R)
         return pl
+
+    def _ndc_args(self, K):
+        """(focal, near) of the NDC warp upstream applies to forward-facing scenes, or None"""
+        return (float(K[0][0]), 1.0) if self.ndc else None
+
+    def _call_render(self, a, K):
+        nd = self._ndc_args(K)
+        if nd is None:
+            call("ctx_render_rays", ctypes.byref(a), stream_ptr(self.device))
+        else:
+            call("ctx_render_rays_ndc", ctypes.byref(a), nd[0], nd[1], stream_ptr(self.device))
 
     # ------------------------------------------------------------------- API
     @torch.no_grad()
@@ -403,7 +440,7 @@ class NerfTrainer:
                         ("depth0", maps_c[3]), ("rgb_map", maps_f[0]), ("disp_map", maps_f[1]), ("acc_map", maps_f[2]),
                         ("depth_map", maps_f[3])):
             setattr(a, name, t.data_ptr())
-        call("ctx_render_rays", ctypes.byref(a), stream_ptr(dev))
+        self._call_render(a, self.K)
         return dict(comp_c=(maps_c[0], maps_c[1], maps_c[2], w_c, maps_c[3]),
                     comp_f=(maps_f[0], maps_f[1], maps_f[2], w_f, maps_f[3]), z_f=z_f, raw_f=raw_f, R=R)
 
@@ -431,8 +468,12 @@ class NerfTrainer:
     def render_view(self, H, W, K, c2w, n_samples=192, sphere=None, near=None, far=None, ray_idx=None):
         """Single-pass render of a view (or of the pixels ``ray_idx`` of it) with the fine network (BASELINE config 4:
         per-ray near/far from the bounding sphere of the normalised mesh, `n_samples` depths per ray, no hierarchical
-        pass).  Maps are [H,W,...] for a whole view, [n,...] for a pixel list."""
+        pass).  Maps are [H,W,...] for a whole view, [n,...] for a pixel list.  An NDC trainer warps the view's rays
+        with its K[0][0]; the sphere interval is metric and is refused there."""
         dev = self.device
+        if self.ndc and sphere is not None:
+            raise CtxNerfError("NerfTrainer.render_view: sphere= gives metric depths; an ndc=True trainer renders "
+                               "between NDC depths near / far")
         f32 = dict(device=dev, dtype=torch.float32)
         c2w_d = torch.as_tensor(c2w, dtype=torch.float32).to(dev).contiguous()
         if ray_idx is not None:
@@ -463,7 +504,7 @@ class NerfTrainer:
                             ("depth_map", depth)):
                 setattr(a, name, t.data_ptr())
             with torch.cuda.device(dev):
-                call("ctx_render_rays", ctypes.byref(a), stream_ptr(dev))
+                self._call_render(a, K)
         if ray_idx is None:
             return dict(rgb_map=rgb.reshape(H, W, 3), disp_map=disp.reshape(H, W), acc_map=acc.reshape(H, W),
                         depth_map=depth.reshape(H, W))

@@ -36,3 +36,15 @@ def multiview_cameras(n_views=8, res=1024, radius=1.5, theta_deg=60.0, fovy=math
     for phi in phis:
         out.append(orbit_camera(res, res, f, radius, 90.0 - theta_deg, float(phi), look_at))
     return out, (look_at[0], look_at[1], look_at[2], 0.6)
+
+
+def forward_facing_camera(H=756, W=1008, focal=815.0, yaw=0.08, pitch=-0.05, eye=(0.05, -0.03, 0.1)):
+    """K and camera-to-world [3,4] of one view of a recentred forward-facing (LLFF) capture: near the origin, looking
+    down -z, slightly turned, so that every ray crosses the NDC near plane z = -1.  Defaults: the size of upstream's
+    LLFF images at factor 4."""
+    K = [[focal, 0.0, 0.5 * W], [0.0, focal, 0.5 * H], [0.0, 0.0, 1.0]]
+    cy, sy, cp, sp = math.cos(yaw), math.sin(yaw), math.cos(pitch), math.sin(pitch)
+    ry = torch.tensor([[cy, 0.0, sy], [0.0, 1.0, 0.0], [-sy, 0.0, cy]], dtype=torch.float64)
+    rx = torch.tensor([[1.0, 0.0, 0.0], [0.0, cp, -sp], [0.0, sp, cp]], dtype=torch.float64)
+    c2w = torch.cat([ry @ rx, torch.tensor(eye, dtype=torch.float64)[:, None]], 1).to(torch.float32)
+    return K, c2w

@@ -112,6 +112,19 @@ int ctx_resample_bwd(const float* bins, int64_t bins_stride, int mid_bins, const
 int ctx_composite_train(const float* raw, const float* z_vals, const float* rays_d, const float* noise,
                         int64_t R, int S, int white_bkgd, const float* target, float loss_scale, float* loss,
                         float* g_raw, float* weights, float* rgb_map, void* stream);
+/* The same with upstream's density noise (raw2outputs: sigma + randn * raw_noise_std) drawn inside the kernel, so
+ * that a captured training step draws fresh noise on every replay without a noise tensor: sample s of ray r gets
+ * noise_std * n, n a standard normal by Box-Muller from Philox4x32-10 with key seed + *seed_dev (seed_dev nullable)
+ * and counter (r, (stream_id << 32) | (s >> 2)), one call for the four samples 4q .. 4q+3 (cos, sin of the first
+ * pair, then of the second).  stream_id >= 2: streams 0 and 1 of a key are the stratified jitter and the
+ * sample_pdf uniforms.  noise_std == 0 runs ctx_composite_train without noise.  ctx_density_noise writes the same
+ * values as a tensor noise [R,S] (a reference for tests; reproduces a step's noise on any host).              */
+int ctx_composite_train_noise(const float* raw, const float* z_vals, const float* rays_d, int64_t R, int S,
+                              int white_bkgd, const float* target, float loss_scale, float* loss, float* g_raw,
+                              float* weights, float* rgb_map, float noise_std, uint64_t seed,
+                              const uint64_t* seed_dev, int stream_id, void* stream);
+int ctx_density_noise(float* noise, int64_t R, int S, float noise_std, uint64_t seed, const uint64_t* seed_dev,
+                      int stream_id, void* stream);
 
 /* ---- coordinate MLP: NeRF2D, src/run_nerf_helpers.py:68-135 (+ the upstream
  * view-direction head kept as comments :86-95, :117-127) ----------------------
@@ -229,6 +242,12 @@ int ctx_step_tick(void* counters, float* loss, void* stream);
 int ctx_adam_step_dev(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n,
                       float lr, float beta1, float beta2, float eps, const void* counters, float weight_decay,
                       float grad_scale, void* stream);
+/* ctx_adam_step_dev with upstream's learning-rate decay (lrate_decay; decay_steps = lrate_decay * 1000 > 0): update
+ * t = counters[1] uses lr * 0.1^(max(t - 2, 0) / decay_steps), the rate upstream's loop has set when its t-th
+ * optimizer.step() runs (the loop sets lrate * 0.1^(global_step / decay_steps) after each step, global_step from 0). */
+int ctx_adam_step_dev_decay(float* params, const float* grads, float* exp_avg, float* exp_avg_sq, int64_t n,
+                            float lr, float beta1, float beta2, float eps, const void* counters, float weight_decay,
+                            float grad_scale, float decay_steps, void* stream);
 
 /* ---- view-weight masks (SURVEY.md 8f row 4): ConTEXTure.create_face_view_map / compare_face_normals_between_views,
  * src/training/trainer.py:155-249 (the reference uses torch_scatter.scatter_max, :227).  face_idx [V,H,W] int64
@@ -279,6 +298,10 @@ typedef struct CtxRenderArgs {
   float *rgb_map, *disp_map, *acc_map, *depth_map;
 } CtxRenderArgs;
 int ctx_render_rays(const CtxRenderArgs* args, void* stream);
+/* the same for forward-facing scenes: the rays are warped to NDC (ndc_rays(H, W, ndc_focal, ndc_near, ...), upstream
+ * uses focal = K[0][0], near = 1) after the view directions are taken from the metric rays; near / far are NDC
+ * depths (upstream: 0 and 1).  sphere must be NULL.                                                              */
+int ctx_render_rays_ndc(const CtxRenderArgs* args, float ndc_focal, float ndc_near, void* stream);
 int ctx_render_args_bytes(void);   /* sizeof(CtxRenderArgs) in the library (layout check for bindings) */
 
 /* ---- gradient all-reduce (SURVEY.md 8b / 8e): the one exchange step of the ray-sharded training step, replacing the
