@@ -41,6 +41,8 @@ struct RaygenParams {
   float* z_vals;    // optional [n, n_samples]
   float* near_far;  // optional [n,2]
   int rays_per_iter;  // rays a warp builds per iteration (power of two, >= rows per pass, <= 32; set by the launcher)
+  // pose stack (raygen_kernel<true>): c2w holds n_views poses pose_stride floats apart, ray_idx global ray ids
+  int n_views, pose_stride;
 };
 
 // z(s) before jitter
@@ -136,6 +138,21 @@ __device__ __forceinline__ void ndc_warp(int H, int W, float focal, float near, 
   ox = n0; oy = n1; oz = n2; dx = e0; dy = e1; dz = e2;
 }
 
+// rotation and origin of a camera-to-world pose, row-major with leading dimension ld
+__device__ __forceinline__ void load_pose(const float* c2w, int ld, float (&rot)[3][3], float (&org)[3]) {
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+#pragma unroll
+    for (int j = 0; j < 3; ++j) rot[k][j] = __ldg(c2w + k * ld + j);
+    org[k] = __ldg(c2w + k * ld + 3);
+  }
+}
+
+// kPoseStack = false: one camera (p.c2w), ray ids are pixel ids y*W + x.  kPoseStack = true: ray ids are global ids
+// view*H*W + y*W + x (upstream's rays_rgb order over [N_train, H, W]) and each lane loads the pose of its own view;
+// everything after the pose load is the one-camera code, so a ray of view v is the ray the one-camera kernel makes
+// with pose v on the same batch row.
+template <bool kPoseStack>
 __global__ void __launch_bounds__(kRayWarps * 32) raygen_kernel(RaygenParams p) {
   // A warp takes 32 rays per iteration.  Phase 1: lane l builds ray r0 + l ONCE (pixel split, the two intrinsics
   // divisions, rotation, norm, view direction, sphere interval) and stores its origin / direction / view direction.
@@ -150,12 +167,7 @@ __global__ void __launch_bounds__(kRayWarps * 32) raygen_kernel(RaygenParams p) 
   const int64_t nwarps = (int64_t)gridDim.x * kRayWarps;
   // camera (uniform loads)
   float rot[3][3], org[3];
-#pragma unroll
-  for (int k = 0; k < 3; ++k) {
-#pragma unroll
-    for (int j = 0; j < 3; ++j) rot[k][j] = __ldg(p.c2w + k * p.c2w_ld + j);
-    org[k] = __ldg(p.c2w + k * p.c2w_ld + 3);
-  }
+  if constexpr (!kPoseStack) load_pose(p.c2w, p.c2w_ld, rot, org);
   const uint64_t seed = p.seed + (p.seed_dev ? *p.seed_dev : 0ull);
   const float zstep = p.n_samples > 1 ? __fdiv_rn(1.0f, (float)(p.n_samples - 1)) : 0.0f;
   const int rpi = p.rays_per_iter;                           // 32 for large launches; fewer so that a small batch
@@ -164,7 +176,13 @@ __global__ void __launch_bounds__(kRayWarps * 32) raygen_kernel(RaygenParams p) 
     float near = p.near, far = p.far;
     if (l32 < rpi && r < p.n_rays) {
       const int64_t pix = p.ray_idx ? p.ray_idx[r] : r;
-      const uint32_t pix32 = (uint32_t)pix;                       // H*W < 2^31 is checked by the launcher
+      uint32_t pix32 = (uint32_t)pix;                             // (n_views*)H*W < 2^31 is checked by the launcher
+      if constexpr (kPoseStack) {
+        const uint32_t hw = (uint32_t)p.H * (uint32_t)p.W;
+        const uint32_t view = min(pix32 / hw, (uint32_t)(p.n_views - 1));   // (clamped: an id past the stack reads no
+        pix32 -= view * hw;                                                   //  memory beyond it)
+        load_pose(p.c2w + (int64_t)view * p.pose_stride, p.c2w_ld, rot, org);
+      }
       const int py = (int)(pix32 / (uint32_t)p.W), px = (int)(pix32 - (uint32_t)py * (uint32_t)p.W);
       const float a = ((float)px - p.cx) / p.fx;
       const float b = -((float)py - p.cy) / p.fy;
@@ -296,19 +314,24 @@ static inline int warp_grid(int64_t rows, int warps_per_cta) {
 
 }  // namespace ctx
 
-extern "C" int ctx_raygen_fwd(int H, int W, float fx, float fy, float cx, float cy, const float* c2w,
-                              int c2w_ld, const int64_t* ray_idx, int64_t n_rays, int use_ndc,
-                              float ndc_focal, float ndc_near, int n_samples, float near, float far,
-                              int lindisp, int perturb, const float* jitter, uint64_t seed,
-                              const uint64_t* seed_dev, int use_sphere, const float* sphere /*host: cx,cy,cz,r*/,
-                              float* rays_o, float* rays_d, float* viewdirs, float* z_vals,
-                              float* near_far, void* stream) {
+namespace ctx {
+
+// the one-camera and the pose-stack launch: same checks, same geometry
+static int launch_raygen(bool pose_stack, int H, int W, float fx, float fy, float cx, float cy, const float* c2w,
+                         int c2w_ld, const int64_t* ray_idx, int64_t n_rays, int use_ndc, float ndc_focal,
+                         float ndc_near, int n_samples, float near, float far, int lindisp, int perturb,
+                         const float* jitter, uint64_t seed, const uint64_t* seed_dev, int use_sphere,
+                         const float* sphere, float* rays_o, float* rays_d, float* viewdirs, float* z_vals,
+                         float* near_far, int n_views, int pose_stride, cudaStream_t stream) {
   if (H < 1 || W < 1 || n_rays < 0 || !c2w || c2w_ld < 4 || n_samples < 0) return CTX_ERR_BAD_ARG;
-  if ((int64_t)H * W >= ((int64_t)1 << 31)) return CTX_ERR_BAD_ARG;   // pixel ids are split with 32-bit arithmetic
+  if (n_views < 1 || pose_stride < 3 * c2w_ld) return CTX_ERR_BAD_ARG;
+  // ray ids are split with 32-bit arithmetic (view, then row and column)
+  if ((int64_t)n_views * H * W >= ((int64_t)1 << 31)) return CTX_ERR_BAD_ARG;
+  if (pose_stack && !ray_idx && n_rays > (int64_t)n_views * H * W) return CTX_ERR_BAD_ARG;
   if (n_rays == 0) return 0;
   if (!rays_o || !rays_d) return CTX_ERR_BAD_ARG;
   if (use_sphere && !sphere) return CTX_ERR_BAD_ARG;
-  ctx::RaygenParams p;
+  RaygenParams p;
   p.H = H; p.W = W; p.fx = fx; p.fy = fy; p.cx = cx; p.cy = cy; p.c2w = c2w; p.c2w_ld = c2w_ld;
   p.ray_idx = ray_idx; p.n_rays = n_rays; p.use_ndc = use_ndc; p.ndc_focal = ndc_focal;
   p.ndc_near = ndc_near; p.n_samples = n_samples; p.near = near; p.far = far; p.lindisp = lindisp;
@@ -317,15 +340,45 @@ extern "C" int ctx_raygen_fwd(int H, int W, float fx, float fy, float cx, float 
   p.sph_cz = use_sphere ? sphere[2] : 0.f; p.sph_r = use_sphere ? sphere[3] : 0.f;
   p.rays_o = rays_o; p.rays_d = rays_d; p.viewdirs = viewdirs;
   p.z_vals = n_samples > 0 ? z_vals : nullptr; p.near_far = near_far;
+  p.n_views = n_views; p.pose_stride = pose_stride;
   {
     const int nl = n_samples > 64 ? 32 : (n_samples > 32 ? 16 : 8);
     int rpi = 32;                                       // halve while the launch would leave SMs without a warp
-    while (rpi > 32 / nl && n_rays < (int64_t)rpi * ctx::kRayWarps * ctx::num_sms() * 2) rpi >>= 1;
+    while (rpi > 32 / nl && n_rays < (int64_t)rpi * kRayWarps * num_sms() * 2) rpi >>= 1;
     p.rays_per_iter = rpi;
   }
-  ctx::raygen_kernel<<<ctx::warp_grid(ctx::ceil_div(n_rays, p.rays_per_iter), ctx::kRayWarps), ctx::kRayWarps * 32, 0,
-                       (cudaStream_t)stream>>>(p);
+  const int grid = warp_grid(ceil_div(n_rays, p.rays_per_iter), kRayWarps);
+  if (pose_stack)
+    raygen_kernel<true><<<grid, kRayWarps * 32, 0, stream>>>(p);
+  else
+    raygen_kernel<false><<<grid, kRayWarps * 32, 0, stream>>>(p);
   CTX_RETURN_LAST();
+}
+
+}  // namespace ctx
+
+extern "C" int ctx_raygen_fwd(int H, int W, float fx, float fy, float cx, float cy, const float* c2w,
+                              int c2w_ld, const int64_t* ray_idx, int64_t n_rays, int use_ndc,
+                              float ndc_focal, float ndc_near, int n_samples, float near, float far,
+                              int lindisp, int perturb, const float* jitter, uint64_t seed,
+                              const uint64_t* seed_dev, int use_sphere, const float* sphere /*host: cx,cy,cz,r*/,
+                              float* rays_o, float* rays_d, float* viewdirs, float* z_vals,
+                              float* near_far, void* stream) {
+  return ctx::launch_raygen(false, H, W, fx, fy, cx, cy, c2w, c2w_ld, ray_idx, n_rays, use_ndc, ndc_focal, ndc_near,
+                            n_samples, near, far, lindisp, perturb, jitter, seed, seed_dev, use_sphere, sphere, rays_o,
+                            rays_d, viewdirs, z_vals, near_far, 1, 3 * c2w_ld, (cudaStream_t)stream);
+}
+
+extern "C" int ctx_raygen_views(int H, int W, float fx, float fy, float cx, float cy, const float* poses,
+                                int c2w_ld, const int64_t* ray_idx, int64_t n_rays, int use_ndc,
+                                float ndc_focal, float ndc_near, int n_samples, float near, float far,
+                                int lindisp, int perturb, const float* jitter, uint64_t seed,
+                                const uint64_t* seed_dev, int use_sphere, const float* sphere /*host: cx,cy,cz,r*/,
+                                float* rays_o, float* rays_d, float* viewdirs, float* z_vals,
+                                float* near_far, int n_views, int pose_stride, void* stream) {
+  return ctx::launch_raygen(true, H, W, fx, fy, cx, cy, poses, c2w_ld, ray_idx, n_rays, use_ndc, ndc_focal, ndc_near,
+                            n_samples, near, far, lindisp, perturb, jitter, seed, seed_dev, use_sphere, sphere, rays_o,
+                            rays_d, viewdirs, z_vals, near_far, n_views, pose_stride, (cudaStream_t)stream);
 }
 
 extern "C" int ctx_stratified_fwd(const float* near, int64_t near_stride, const float* far,

@@ -26,6 +26,11 @@ _SIGNATURES = {
     "ctx_raygen_fwd": (c_int, [c_int, c_int, c_float, c_float, c_float, c_float, P, c_int, P, c_int64,
                                c_int, c_float, c_float, c_int, c_float, c_float, c_int, c_int, P,
                                c_uint64, P, c_int, P, P, P, P, P, P, P]),
+    "ctx_raygen_views": (c_int, [c_int, c_int, c_float, c_float, c_float, c_float, P, c_int, P, c_int64,
+                                 c_int, c_float, c_float, c_int, c_float, c_float, c_int, c_int, P,
+                                 c_uint64, P, c_int, P, P, P, P, P, P, c_int, c_int, P]),
+    "ctx_draw_rays": (c_int, [P, c_int, c_int, c_int, c_int64, c_int, c_int, c_int, c_int, c_int, c_int, c_uint64, P,
+                              P, P, P]),
     "ctx_stratified_fwd": (c_int, [P, c_int64, P, c_int64, c_int64, c_int, c_int, c_int, P, c_uint64, P, P]),
     "ctx_ndc_fwd": (c_int, [c_int, c_int, c_float, c_float, P, P, c_int64, P, P, P]),
     "ctx_ndc_bwd": (c_int, [c_int, c_int, c_float, c_float, P, P, P, P, c_int64, P, P, P]),

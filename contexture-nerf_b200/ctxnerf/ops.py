@@ -218,7 +218,10 @@ def resample_raw(bins, weights, n_samples, det=True, u=None, cdf=None, seed=0):
 def raygen(H, W, K, c2w, *, device=None, ray_idx=None, ndc=None, n_samples=0, near=0.0, far=1.0,
            lindisp=False, perturb=False, jitter=None, seed=None, sphere=None, want_viewdirs=False,
            want_near_far=False, seed_dev=None, out=None):
-    """Fused get_rays (+ndc) (+viewdirs) (+stratified z_vals).  Returns a dict."""
+    """Fused get_rays (+ndc) (+viewdirs) (+stratified z_vals).  Returns a dict.
+
+    ``c2w`` is one pose [3|4, 4] (``ray_idx``: pixel ids y*W + x) or a stack [N, 3|4, 4] (``ctx_raygen_views``:
+    ``ray_idx`` holds global ids view*H*W + y*W + x, None = all N*H*W rays in that order)."""
     if torch.is_tensor(c2w):
         dev = c2w.device if c2w.is_cuda else torch.device(device or "cuda")
         c2w_d = c2w.to(device=dev, dtype=torch.float32)
@@ -230,12 +233,16 @@ def raygen(H, W, K, c2w, *, device=None, ray_idx=None, ndc=None, n_samples=0, ne
         c2w_d = c2w_d.to(dev)
     c2w_d = c2w_d.contiguous()
     ld = c2w_d.shape[-1]
+    stack = c2w_d.dim() == 3
+    if c2w_d.dim() not in (2, 3) or tuple(c2w_d.shape[-2:]) not in ((3, 4), (4, 4)):
+        raise _lib.CtxNerfError(f"raygen: c2w must be [3|4, 4] or [N, 3|4, 4], got {tuple(c2w_d.shape)}")
+    n_views = c2w_d.shape[0] if stack else 1
     fx, fy, cx, cy = float(K[0][0]), float(K[1][1]), float(K[0][2]), float(K[1][2])
     if ray_idx is not None:
         ray_idx = ray_idx.to(device=dev, dtype=torch.int64).contiguous()
         n = ray_idx.numel()
     else:
-        n = H * W
+        n = n_views * H * W
     if out is not None:          # caller-owned (static) outputs: (rays_o, rays_d, viewdirs, z_vals)
         o, d, v, z = out
     else:
@@ -250,13 +257,39 @@ def raygen(H, W, K, c2w, *, device=None, ray_idx=None, ndc=None, n_samples=0, ne
     sph = (ctypes.c_float * 4)(*[float(s) for s in sphere]) if sphere is not None else None
     use_ndc, nfoc, nnear = (1, float(ndc[0]), float(ndc[1])) if ndc is not None else (0, 0.0, 0.0)
     jitter = _f32c(jitter)
+    args = (int(H), int(W), fx, fy, cx, cy, ptr(c2w_d), int(ld), ptr(ray_idx), n, use_ndc, nfoc, nnear,
+            int(n_samples), float(near), float(far), int(lindisp), int(bool(perturb)), ptr(jitter), int(seed or 0),
+            ptr(seed_dev), int(sphere is not None), ctypes.cast(sph, ctypes.c_void_p) if sph is not None else None,
+            ptr(o), ptr(d), ptr(v), ptr(z), ptr(nf))
     with torch.cuda.device(dev):
-        call("ctx_raygen_fwd", int(H), int(W), fx, fy, cx, cy, ptr(c2w_d), int(ld), ptr(ray_idx), n, use_ndc,
-             nfoc, nnear, int(n_samples), float(near), float(far), int(lindisp), int(bool(perturb)),
-             ptr(jitter), int(seed or 0), ptr(seed_dev), int(sphere is not None),
-             ctypes.cast(sph, ctypes.c_void_p) if sph is not None else None,
-             ptr(o), ptr(d), ptr(v), ptr(z), ptr(nf), stream_ptr(dev))
+        if stack:
+            call("ctx_raygen_views", *args, n_views, int(c2w_d.stride(0)), stream_ptr(dev))
+        else:
+            call("ctx_raygen_fwd", *args, stream_ptr(dev))
     return {"rays_o": o, "rays_d": d, "viewdirs": v, "z_vals": z, "near_far": nf}
+
+
+def draw_rays(n_views, H, W, R, counters, *, images=None, mode=0, precrop_iters=0, crop=(0, 0), rank=0, world=1,
+              seed=0, out=None):
+    """Upstream train()'s ray batch drawn on the device (``ctx_draw_rays``): R global ray ids view*H*W + y*W + x and,
+    with ``images`` [n_views, H, W, 3] fp32, their target colours.  ``counters`` is the step state ctx_step_tick
+    advances ([0] Philox offset, [1] step count).  mode 0: one view per step, R distinct pixels of it (from the centre
+    crop of half-extents ``crop`` = (dH, dW) while the step count is below ``precrop_iters``); mode 1: an epoch stream
+    over every ray.  Returns (ray_idx [R] int64, target [R,3] or None)."""
+    _need_cuda(counters, images)
+    dev = counters.device
+    if images is not None and (images.dtype != torch.float32 or not images.is_contiguous()):
+        raise _lib.CtxNerfError("draw_rays: images must be a contiguous fp32 [n_views, H, W, 3] tensor")
+    if out is not None:          # caller-owned (static) outputs: the captured training step
+        idx, tgt = out
+    else:
+        idx = torch.empty(R, device=dev, dtype=torch.int64)
+        tgt = torch.empty(R, 3, device=dev, dtype=torch.float32) if images is not None else None
+    with torch.cuda.device(dev):
+        call("ctx_draw_rays", ptr(images), int(n_views), int(H), int(W), int(R), int(mode), int(precrop_iters),
+             int(crop[0]), int(crop[1]), int(rank), int(world), int(seed), ptr(counters), ptr(idx), ptr(tgt),
+             stream_ptr(dev))
+    return idx, tgt
 
 
 def stratified(near, far, n_samples, lindisp=False, perturb=False, jitter=None, seed=None):

@@ -41,10 +41,11 @@ def _env_int(name, default):
 class _Plan:
     """Static device buffers of the training step for one batch size R."""
 
-    def __init__(self, tr: "NerfTrainer", R: int):
+    def __init__(self, tr: "NerfTrainer", R: int, draw: bool = False):
         dev, S, Sf = tr.device, tr.N_samples, tr.N_samples + tr.N_importance
         f32 = dict(device=dev, dtype=torch.float32)
         self.R = R
+        self.draw = draw           # True: the step draws idx / target itself (ctx_draw_rays); False: the caller's batch
         self.idx = torch.zeros(R, device=dev, dtype=torch.int64)
         self.target = torch.zeros(R, 3, **f32)
         self.o, self.d, self.v = (torch.empty(R, 3, **f32) for _ in range(3))
@@ -68,8 +69,18 @@ class _Plan:
 
 
 class NerfTrainer:
-    """Upstream nerf-pytorch's training step for one camera.  The defaults are its Blender recipe; its forward-facing
-    (LLFF) recipe is ``ndc=True, near=0, far=1, raw_noise_std=1.0, lrate_decay=250, white_bkgd=False``:
+    """Upstream nerf-pytorch's training step on one camera or a set of posed images.  The defaults are its Blender
+    recipe; its forward-facing (LLFF) recipe is ``ndc=True, near=0, far=1, raw_noise_std=1.0, lrate_decay=250,
+    white_bkgd=False, no_batching=False``:
+
+    * ``c2w``: one pose [3|4, 4] or a stack [N, 3|4, 4] (one K for every view, as upstream).  ``step`` takes global ray
+      ids view*H*W + y*W + x (with one pose, the pixel ids y*W + x).  The stack lives on the device as ``poses``;
+      ``c2w`` is its first pose.
+    * ``images`` [N, H, W, 3] (float in [0, 1], or uint8), the training images of the poses, kept on the device as
+      fp32.  ``step_random(N_rand)`` then draws each step's batch on the device, inside the captured step, as upstream's
+      loop does: ``no_batching=True`` takes one random image per step and N_rand distinct pixels of it (from the
+      centre crop ``precrop_frac`` for the first ``precrop_iters`` steps); ``no_batching=False`` walks a stream over
+      every ray of every image, reshuffled each epoch (csrc/raybatch.cu gives the construction).
 
     * ``ndc``: rays are warped by ``ndc_rays(H, W, K[0][0], 1., ...)`` after the view directions are taken, so
       near / far are NDC depths.  Training, ``render`` and ``render_view`` all use the warped rays.
@@ -82,7 +93,30 @@ class NerfTrainer:
 
     def __init__(self, H, W, K, c2w, near=2.0, far=6.0, N_samples=64, N_importance=128, perturb=1.0,
                  white_bkgd=True, lindisp=False, lr=5e-4, betas=(0.9, 0.999), eps=1e-8, device=None, seed=0,
-                 multires=10, multires_views=4, ndc=False, raw_noise_std=0.0, lrate_decay=0):
+                 multires=10, multires_views=4, ndc=False, raw_noise_std=0.0, lrate_decay=0, images=None,
+                 no_batching=True, precrop_iters=0, precrop_frac=0.5):
+        c2w_h = torch.as_tensor(c2w, dtype=torch.float32)
+        if c2w_h.dim() not in (2, 3) or tuple(c2w_h.shape[-2:]) not in ((3, 4), (4, 4)):
+            raise CtxNerfError(f"NerfTrainer: c2w must be [3|4, 4] or a stack [N, 3|4, 4], got {tuple(c2w_h.shape)}")
+        n_views = c2w_h.shape[0] if c2w_h.dim() == 3 else 1
+        if n_views < 1:
+            raise CtxNerfError("NerfTrainer: the pose stack is empty")
+        if n_views * H * W >= 2 ** 31:
+            raise CtxNerfError("NerfTrainer: N*H*W must stay below 2^31 (global ray ids are split in 32 bits)")
+        if images is not None:
+            shape = tuple(images.shape)
+            if shape != (n_views, H, W, 3):
+                raise CtxNerfError(f"NerfTrainer: images must be [N, H, W, 3] = {(n_views, H, W, 3)} for {n_views} "
+                                   f"pose(s) of {H}x{W}, got {shape}")
+        if not (0.0 < precrop_frac <= 1.0):
+            raise CtxNerfError("NerfTrainer: precrop_frac must lie in (0, 1]")
+        if not precrop_iters >= 0:
+            raise CtxNerfError("NerfTrainer: precrop_iters must be >= 0")
+        if precrop_iters > 0 and not no_batching:
+            raise CtxNerfError("NerfTrainer: precrop_iters crops the one image a step draws from (no_batching=True)")
+        crop = (int(H // 2 * precrop_frac), int(W // 2 * precrop_frac))     # upstream's dH, dW
+        if precrop_iters > 0 and min(crop) < 1:
+            raise CtxNerfError(f"NerfTrainer: the centre crop of precrop_frac={precrop_frac} is empty at {H}x{W}")
         if not raw_noise_std >= 0.0:
             raise CtxNerfError("NerfTrainer: raw_noise_std must be >= 0")
         if not lrate_decay >= 0:
@@ -90,7 +124,15 @@ class NerfTrainer:
         self.device = torch.device(device if device is not None else ("cuda", torch.cuda.current_device()))
         dev = self.device
         self.H, self.W, self.K = H, W, K
-        self.c2w = torch.as_tensor(c2w, dtype=torch.float32).to(dev).contiguous()
+        self.n_views = n_views
+        if c2w_h.dim() == 3:
+            self.poses = c2w_h.to(dev).contiguous()
+            self.c2w = self.poses[0]
+        else:
+            self.c2w = c2w_h.to(dev).contiguous()
+            self.poses = self.c2w[None]
+        self.no_batching, self.precrop_iters, self.precrop_frac = bool(no_batching), int(precrop_iters), precrop_frac
+        self._crop = crop
         self.near, self.far = float(near), float(far)
         self.N_samples, self.N_importance = int(N_samples), int(N_importance)
         self.perturb, self.white_bkgd, self.lindisp = float(perturb), bool(white_bkgd), bool(lindisp)
@@ -102,6 +144,8 @@ class NerfTrainer:
         in_pts, in_views = 3 * (1 + 2 * multires), 3 * (1 + 2 * multires_views)
         self.coarse = NeRF(input_ch=in_pts, input_ch_views=in_views).to(dev)
         self.fine = NeRF(input_ch=in_pts, input_ch_views=in_views).to(dev)
+        # key of the epoch stream (no_batching=False): from the same seed, so every rank walks the same permutation
+        self._stream_key = ops.new_seed() if images is not None and not no_batching else 0
         torch.random.set_rng_state(st)
         for net in (self.coarse, self.fine):
             net.L_pts, net.L_dirs = multires, multires_views
@@ -123,7 +167,13 @@ class NerfTrainer:
         # device-side step state: [0] Philox seed offset, [1] Adam step count (ctx_step_tick advances both)
         self._ctr = torch.zeros(2, device=dev, dtype=torch.int64)
         # the Philox base seed comes from torch's generator: torch.manual_seed makes a training run reproducible
-        self._seed0 = ops.new_seed() if self.perturb > 0.0 or self.raw_noise_std > 0.0 else 0
+        # (a trainer with images keys its per-step image and pixel draw with it too)
+        self._seed0 = ops.new_seed() if self.perturb > 0.0 or self.raw_noise_std > 0.0 or images is not None else 0
+        self.images = None
+        if images is not None:
+            im = torch.as_tensor(images)
+            im = im.to(dev).float().div_(255.0) if im.dtype == torch.uint8 else im.to(dev, dtype=torch.float32)
+            self.images = im.contiguous()
         # bf16 weight streams of both networks: trainer-owned static buffers, re-packed after every Adam update
         self._pk = {}
         for net in (self.coarse, self.fine):
@@ -234,9 +284,15 @@ class NerfTrainer:
         jit = self.perturb > 0.0
         main = torch.cuda.current_stream(dev)
         call("ctx_step_tick", ptr(self._ctr), ptr(self._loss), stream_ptr(dev))
+        if pl.draw:
+            ops.draw_rays(self.n_views, self.H, self.W, R, self._ctr, images=self.images,
+                          mode=0 if self.no_batching else 1, precrop_iters=self.precrop_iters, crop=self._crop,
+                          rank=self.rank, world=self.world_size,
+                          seed=self._seed0 if self.no_batching else self._stream_key, out=(pl.idx, pl.target))
         self.bucket.zero_grad()
-        ops.raygen(self.H, self.W, self.K, self.c2w, ray_idx=pl.idx, n_samples=S, near=self.near, far=self.far,
-                   lindisp=self.lindisp, perturb=jit, seed=self._seed0, seed_dev=self._ctr if jit else None,
+        # one pose: ctx_raygen_fwd; a stack: ctx_raygen_views (each ray the pose of its view)
+        ops.raygen(self.H, self.W, self.K, self.c2w if self.n_views == 1 else self.poses, ray_idx=pl.idx, n_samples=S,
+                   near=self.near, far=self.far, lindisp=self.lindisp, perturb=jit, seed=self._seed0, seed_dev=self._ctr if jit else None,
                    ndc=self._ndc_args(self.K), want_viewdirs=True, out=(pl.o, pl.d, pl.v, pl.z_c))
         rays_c, rays_f = (pl.o, pl.d, pl.v, pl.z_c), (pl.o, pl.d, pl.v, pl.z_f)
         self._timed("mlp_fwd_coarse", lambda: self._fwd(self.coarse, rays_c, Pc, pl.raw_c, pl.acts_c))
@@ -284,10 +340,13 @@ class NerfTrainer:
             call("ctx_adam_step_dev", *args, stream_ptr(dev))
         self._repack()
 
-    def _plan(self, R: int) -> _Plan:
-        pl = self._plans.get(R)
+    def _plan(self, R: int, draw: bool = False) -> _Plan:
+        """Static buffers (and graphs) of one batch size: ``_plans[R]`` for the caller's batches, ``_plans[(R, "draw")]``
+        for batches the step draws itself."""
+        key = (R, "draw") if draw else R
+        pl = self._plans.get(key)
         if pl is None:
-            pl = self._plans[R] = _Plan(self, R)
+            pl = self._plans[key] = _Plan(self, R, draw)
         return pl
 
     def _ndc_args(self, K):
@@ -321,6 +380,29 @@ class NerfTrainer:
             pl = self._plan(R)
             pl.idx.copy_(ray_idx.reshape(-1), non_blocking=True)
             pl.target.copy_(target.reshape(R, 3), non_blocking=True)     # (casts a non-fp32 target)
+            self._run(pl, optimizer_step)
+        return self._loss
+
+    @torch.no_grad()
+    def step_random(self, N_rand: int, optimizer_step: bool = True) -> torch.Tensor:
+        """One training step on a batch of N_rand rays drawn on the device from the training images, as upstream's
+        loop draws it (``no_batching``, ``precrop_iters``, ``precrop_frac``); returns the loss (device scalar).  The
+        draw is part of the step: a captured step draws a fresh batch on every replay, and the batch of the last step
+        is in ``_plans[(N_rand, "draw")].idx / .target``.  Under several ranks each rank draws its own share."""
+        if self.images is None:
+            raise CtxNerfError("NerfTrainer.step_random draws from the training images: build the trainer with images=")
+        R = int(N_rand)
+        if R < 1:
+            raise CtxNerfError("NerfTrainer.step_random: N_rand must be >= 1")
+        if self.no_batching:
+            dom = self.H * self.W
+            if self.precrop_iters > 0:
+                dom = min(dom, 4 * self._crop[0] * self._crop[1])
+            if R > dom:
+                raise CtxNerfError(f"NerfTrainer.step_random: N_rand={R} distinct pixels of one image, but the "
+                                   f"{'centre crop' if dom < self.H * self.W else 'image'} has {dom}")
+        with torch.cuda.device(self.device):
+            pl = self._plan(R, draw=True)
             self._run(pl, optimizer_step)
         return self._loss
 
@@ -403,7 +485,7 @@ class NerfTrainer:
         return done     # loss_pinned is valid once this event has completed
 
     # ------------------------------------------------------------ inference
-    def _render(self, ray_idx, perturb, seed=0, max_sms=0):
+    def _render(self, ray_idx, perturb, seed=0, max_sms=0, c2w=None):
         """Forward-only coarse+fine render of the given pixels (None = the whole image): dynamic shapes, fresh
         outputs; shares the trainer's packed weights.  ONE C-ABI call: ctx_render_rays (csrc/render.cu) enqueues
         raygen -> MLP -> raw2outputs -> sample_pdf + merge -> MLP -> raw2outputs."""
@@ -424,7 +506,12 @@ class NerfTrainer:
         a = _lib.CtxRenderArgs()
         a.H, a.W = self.H, self.W
         a.fx, a.fy, a.cx, a.cy = (float(self.K[0][0]), float(self.K[1][1]), float(self.K[0][2]), float(self.K[1][2]))
-        a.c2w, a.c2w_ld = self.c2w.data_ptr(), self.c2w.stride(0)
+        pose = self.c2w
+        if c2w is not None:
+            pose = torch.as_tensor(c2w, dtype=torch.float32).to(dev).contiguous()
+            if tuple(pose.shape) not in ((3, 4), (4, 4)):
+                raise CtxNerfError(f"NerfTrainer.render: c2w must be one pose [3|4, 4], got {tuple(pose.shape)}")
+        a.c2w, a.c2w_ld = pose.data_ptr(), pose.stride(0)
         a.ray_idx, a.n_rays = (None if ray_idx is None else ray_idx.data_ptr()), R
         a.near, a.far, a.lindisp, a.perturb = self.near, self.far, int(self.lindisp), int(bool(perturb))
         a.seed, a.seed_dev, a.sphere = int(seed), None, None
@@ -456,11 +543,13 @@ class NerfTrainer:
         return rgb, disp, acc, w, depth
 
     @torch.no_grad()
-    def render(self, ray_idx: Optional[torch.Tensor] = None):
-        """Inference render of the given pixels (None = the whole H x W image).  Deterministic, as upstream's
-        render_kwargs_test (perturb=False, raw_noise_std=0): linspace depths and det=True importance sampling."""
+    def render(self, ray_idx: Optional[torch.Tensor] = None, c2w=None):
+        """Inference render of the given pixels (None = the whole H x W image) of the pose ``c2w`` [3|4, 4] (None = the
+        first training pose), with the trainer's K: held-out test poses render through here.  Deterministic, as
+        upstream's render_kwargs_test (perturb=False, raw_noise_std=0): linspace depths and det=True importance
+        sampling."""
         with torch.cuda.device(self.device):
-            fwd = self._render(ray_idx, perturb=False)
+            fwd = self._render(ray_idx, perturb=False, c2w=c2w)
         rgb, disp, acc, _, depth = fwd["comp_f"]
         return dict(rgb_map=rgb, disp_map=disp, acc_map=acc, depth_map=depth, rgb0=fwd["comp_c"][0])
 

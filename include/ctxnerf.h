@@ -57,6 +57,36 @@ int ctx_raygen_fwd(int H, int W, float fx, float fy, float cx, float cy, const f
 /* seed_dev (nullable, here and in ctx_resample_fwd): a DEVICE counter added to `seed` inside the kernel, so that a
  * captured CUDA graph of the training step draws fresh Philox numbers on every replay (ctx_adam_step_dev bumps it). */
 
+/* The same over a stack of poses (multi-view training): poses = n_views camera-to-world matrices pose_stride floats
+ * apart (12 for [N,3,4], 16 for [N,4,4]), rows c2w_ld apart; ray_idx holds GLOBAL ray ids view*H*W + y*W + x
+ * (upstream's rays_rgb order over [N_train, H, W]; NULL = ids 0..n_rays-1), n_views*H*W < 2^31.  Each ray takes the
+ * pose of its view; a ray of view v is the ray ctx_raygen_fwd makes with pose v on the same batch row, bit for bit
+ * (jitter included: it is keyed by the batch row).  One K for every view.                                        */
+int ctx_raygen_views(int H, int W, float fx, float fy, float cx, float cy, const float* poses,
+                     int c2w_ld, const int64_t* ray_idx, int64_t n_rays, int use_ndc,
+                     float ndc_focal, float ndc_near, int n_samples, float near, float far,
+                     int lindisp, int perturb, const float* jitter, uint64_t seed,
+                     const uint64_t* seed_dev, int use_sphere, const float* sphere, float* rays_o,
+                     float* rays_d, float* viewdirs, float* z_vals, float* near_far, int n_views, int pose_stride,
+                     void* stream);
+
+/* ---- training ray batches drawn on the device: upstream run_nerf.py train()'s samplers -------------------------
+ * ray_idx [R] int64 <- R global ray ids; target (nullable, [R,3]) <- images[v, y, x, :] (images [n_views,H,W,3] fp32,
+ * nullable when target is NULL).  Both modes sample without replacement through a keyed Feistel permutation
+ * evaluated pointwise (construction in csrc/raybatch.cu).  counters = ctx_step_tick's pair ([0] Philox offset, [1]
+ * step count t, 1 on the first step).
+ * mode 0 (no_batching=True): one view per step, drawn uniformly with key seed + counters[0] on Philox stream 4 (rank
+ *   in the counter), and R distinct pixels of it; while t < precrop_iters only from upstream's centre crop, rows
+ *   [H/2 - crop_dh, H/2 + crop_dh) x cols [W/2 - crop_dw, W/2 + crop_dw) (crop_dh = int(H//2 * precrop_frac)).
+ * mode 1 (no_batching=False): position ((t-1)*world + rank)*R + r of an epoch stream over all n_views*H*W rays, each
+ *   epoch a permutation keyed by (seed, epoch): seed must be the same on every rank.  A batch that straddles an epoch
+ *   boundary takes the tail of one epoch and the head of the next.  precrop_iters must be 0.
+ * Bad arguments (before any launch): null ray_idx / counters, R < 0, mode 0 with R above the (cropped) pixel count,
+ * an empty crop, rank outside [0, world), n_views*H*W >= 2^31.                                                  */
+int ctx_draw_rays(const float* images, int n_views, int H, int W, int64_t R, int mode, int precrop_iters,
+                  int crop_dh, int crop_dw, int rank, int world, uint64_t seed, const void* counters,
+                  int64_t* ray_idx, float* target, void* stream);
+
 /* z_vals [R,S] from per-ray near/far (ray_batch[:,6], ray_batch[:,7] upstream) */
 int ctx_stratified_fwd(const float* near, int64_t near_stride, const float* far,
                        int64_t far_stride, int64_t R, int S, int lindisp, int perturb,
