@@ -73,6 +73,8 @@ _SIGNATURES = {
     "ctx_render_rays": (c_int, [P, P]),
     "ctx_render_rays_ndc": (c_int, [P, c_float, c_float, P]),
     "ctx_render_args_bytes": (c_int, []),
+    "ctx_image_metrics": (c_int, [P, P, c_int, c_int, c_int, c_int, P, P, P, P]),
+    "ctx_image_metrics_partials": (c_int64, [c_int, c_int, c_int]),
     "ctx_comm_load": (c_int, [ctypes.c_char_p]),
     "ctx_comm_version": (c_int, []),
     "ctx_comm_last_error": (ctypes.c_char_p, []),
@@ -168,7 +170,7 @@ def check(code: int, what: str) -> None:
 
 
 # kernels launched per ABI call (bench.py reports the total as gpu_launches)
-KERNELS_PER_CALL = {"ctx_mlp_bwd": 3, "ctx_mlp_wgrad": 2, "ctx_mlp_wgrad_ex": 2, "ctx_composite_train": 2, "ctx_composite_train_noise": 2, "ctx_render_rays": 6, "ctx_render_rays_ndc": 6, "ctx_allreduce": 0, "ctx_comm_load": 0, "ctx_comm_unique_id": 0, "ctx_comm_init": 0, "ctx_comm_destroy": 0}     # (the view-direction wgrad also runs a small post kernel: +1, counted by the callers that know the net)
+KERNELS_PER_CALL = {"ctx_mlp_bwd": 3, "ctx_mlp_wgrad": 2, "ctx_mlp_wgrad_ex": 2, "ctx_composite_train": 2, "ctx_composite_train_noise": 2, "ctx_render_rays": 6, "ctx_render_rays_ndc": 6, "ctx_image_metrics": 2, "ctx_allreduce": 0, "ctx_comm_load": 0, "ctx_comm_unique_id": 0, "ctx_comm_init": 0, "ctx_comm_destroy": 0}     # (the view-direction wgrad also runs a small post kernel: +1, counted by the callers that know the net)
 launch_count = 0
 
 

@@ -339,3 +339,35 @@ class _Ndc(torch.autograd.Function):
 
 def ndc(H, W, focal, near, rays_o, rays_d):
     return _Ndc.apply(H, W, focal, near, rays_o, rays_d)
+
+
+# ----------------------------------------------------------------- metrics ---
+def image_metrics(pred: torch.Tensor, target: torch.Tensor):
+    """Reconstruction metrics of rendered images (``ctx_image_metrics``): ``pred`` [B,H,W,3] or [H,W,3] fp32,
+    ``target`` of the same shape, fp32 or uint8 (read as u8 / 255), on the same device.  Returns ``(mse, psnr,
+    ssim)``, fp64 device tensors [B] (B = 1 for one image): upstream's img2mse and mse2psnr (psnr = -10 log10(mse),
+    +inf at mse 0) and SSIM as mip-NeRF's compute_ssim (11-tap Gaussian window, sigma 1.5, max_val 1; H, W >= 11).
+    Neither image is clamped."""
+    _need_cuda(pred, target)
+    if pred.dtype != torch.float32:
+        raise _lib.CtxNerfError(f"image_metrics: pred must be fp32, got {pred.dtype}")
+    if target.dtype not in (torch.float32, torch.uint8):
+        raise _lib.CtxNerfError(f"image_metrics: target must be fp32 or uint8, got {target.dtype}")
+    if pred.dim() not in (3, 4) or pred.shape[-1] != 3 or tuple(target.shape) != tuple(pred.shape):
+        raise _lib.CtxNerfError(f"image_metrics: pred and target must both be [B,H,W,3] or [H,W,3], got "
+                                f"{tuple(pred.shape)} and {tuple(target.shape)}")
+    if target.device != pred.device:
+        raise _lib.CtxNerfError(f"image_metrics: pred is on {pred.device}, target on {target.device}")
+    B, H, W = (1, *pred.shape[:2]) if pred.dim() == 3 else pred.shape[:3]
+    if min(H, W) < 11:
+        raise _lib.CtxNerfError(f"image_metrics: SSIM's 11-tap window needs H, W >= 11, got {H}x{W}")
+    dev = pred.device
+    pred, target = pred.contiguous(), target.contiguous()
+    mse = torch.empty(B, device=dev, dtype=torch.float64)
+    ssim = torch.empty(B, device=dev, dtype=torch.float64)
+    if B > 0:
+        partials = torch.empty(int(_lib.lib().ctx_image_metrics_partials(B, H, W)), device=dev, dtype=torch.float64)
+        with torch.cuda.device(dev):
+            call("ctx_image_metrics", ptr(pred), ptr(target), int(target.dtype == torch.uint8), B, H, W, ptr(mse),
+                 ptr(ssim), ptr(partials), stream_ptr(dev))
+    return mse, mse.log10().mul_(-10.0), ssim

@@ -554,6 +554,51 @@ class NerfTrainer:
         return dict(rgb_map=rgb, disp_map=disp, acc_map=acc, depth_map=depth, rgb0=fwd["comp_c"][0])
 
     @torch.no_grad()
+    def evaluate(self, c2w, images):
+        """Test-split metrics, as NeRF results are reported: each pose of ``c2w`` [N, 3|4, 4] renders through
+        ``render(c2w=pose)`` (deterministic, with the trainer's K, NDC warp and ``white_bkgd``) and is compared with its
+        image of ``images`` [N, H, W, 3] (fp32 in [0, 1] or uint8, on the host or the device, at the trainer's H x W) by
+        ``ops.image_metrics``.  Returns ``dict(mse=, psnr=, ssim=)``, CPU fp64 tensors [N], one entry per pose:
+        upstream's img2mse and mse2psnr, and SSIM as mip-NeRF's compute_ssim.
+
+        The targets must already be composited the way the trainer renders, e.g. onto white for ``white_bkgd=True``
+        (upstream's Blender loader does ``rgb * alpha + (1 - alpha)``): neither image is clamped or blended here.  A
+        uint8 stack stays uint8 on the device (the kernel converts it); a host stack is copied to the device once, up
+        front, and the results come back with one host synchronisation at the end.
+
+        Under several ranks every rank calls ``evaluate`` with the same arguments: rank r renders the views
+        v = r mod world, and one all-reduce of the [3, N] results (zero outside a rank's views, so the sum is exact)
+        gives every rank the single-process vectors bit for bit.  The training state is left as it was: the step
+        counters, the loss, the Adam moments, the weights and their packed images, the captured step graphs and torch's
+        random number generator."""
+        P = torch.as_tensor(c2w, dtype=torch.float32)
+        if P.dim() != 3 or tuple(P.shape[1:]) not in ((3, 4), (4, 4)):
+            raise CtxNerfError(f"NerfTrainer.evaluate: c2w must be a stack [N, 3|4, 4], got {tuple(P.shape)}")
+        images = torch.as_tensor(images)
+        N = P.shape[0]
+        if tuple(images.shape) != (N, self.H, self.W, 3):
+            raise CtxNerfError(f"NerfTrainer.evaluate: images must be [N, H, W, 3] = {(N, self.H, self.W, 3)} for {N} "
+                               f"pose(s) of the trainer's {self.H}x{self.W}, got {tuple(images.shape)}")
+        if images.dtype not in (torch.float32, torch.uint8):
+            raise CtxNerfError(f"NerfTrainer.evaluate: images must be fp32 or uint8, got {images.dtype}")
+        if N == 0:
+            empty = torch.empty(0, dtype=torch.float64)
+            return dict(mse=empty, psnr=empty.clone(), ssim=empty.clone())
+        dev = self.device
+        with torch.cuda.device(dev):
+            vals = torch.zeros(3, N, device=dev, dtype=torch.float64)
+            poses = P.to(dev)
+            targets = images[self.rank::self.world_size].to(dev)
+            for i, v in enumerate(range(self.rank, N, self.world_size)):
+                rgb = self.render(c2w=poses[v])["rgb_map"].view(self.H, self.W, 3)
+                vals[:, v] = torch.cat(ops.image_metrics(rgb, targets[i]))
+            if self.world_size > 1:
+                import torch.distributed as dist
+                dist.all_reduce(vals)
+            out = vals.cpu()
+        return dict(mse=out[0], psnr=out[1], ssim=out[2])
+
+    @torch.no_grad()
     def render_view(self, H, W, K, c2w, n_samples=192, sphere=None, near=None, far=None, ray_idx=None):
         """Single-pass render of a view (or of the pixels ``ray_idx`` of it) with the fine network (BASELINE config 4:
         per-ray near/far from the bounding sphere of the normalised mesh, `n_samples` depths per ray, no hierarchical

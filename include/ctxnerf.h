@@ -334,6 +334,23 @@ int ctx_render_rays(const CtxRenderArgs* args, void* stream);
 int ctx_render_rays_ndc(const CtxRenderArgs* args, float ndc_focal, float ndc_near, void* stream);
 int ctx_render_args_bytes(void);   /* sizeof(CtxRenderArgs) in the library (layout check for bindings) */
 
+/* ---- evaluation metrics of a test split: upstream img2mse / mse2psnr (src/run_nerf_helpers.py:9-10) and SSIM as
+ * the compute_ssim of mip-NeRF / MultiNeRF (max_val = 1; restated in csrc/metrics.cu and oracle/image_metrics.py).
+ * Per-image reconstruction metrics of a batch of B images.
+ * pred: [B,H,W,3] fp32 device.
+ * target: [B,H,W,3] device, fp32 (target_u8 == 0) or uint8 (target_u8 == 1, read as u8 / 255.0f, IEEE division).
+ * mse (nullable, [B] double): mean over H*W*3 of (pred - target)^2.  The difference is formed in fp32; squares and
+ *   sums are in fp64.
+ * ssim (nullable, [B] double): mean of the SSIM map (11-tap Gaussian window, sigma 1.5, valid mode) over the three
+ *   channels and the (H-10) x (W-10) positions.  Neither image is clamped.
+ * partials: caller-owned device workspace of ctx_image_metrics_partials(B, H, W) doubles.
+ * Deterministic (no floating-point atomics), and an image gives the same bits whatever the batch around it.
+ * Bad arguments: B < 0, H < 1, W < 1, target_u8 outside {0, 1}, ssim != NULL with min(H, W) < 11, a null pred /
+ * target / partials when B > 0.  B == 0 returns 0.                                                               */
+int ctx_image_metrics(const float* pred, const void* target, int target_u8, int B, int H, int W,
+                      double* mse, double* ssim, double* partials, void* stream);
+int64_t ctx_image_metrics_partials(int B, int H, int W);   /* -1 for B < 0, H < 1 or W < 1 */
+
 /* ---- gradient all-reduce (SURVEY.md 8b / 8e): the one exchange step of the ray-sharded training step, replacing the
  * reduce-add of nn.DataParallel (src/training/trainer.py:134-135).  NCCL is opened at run time (dlopen; `path`
  * nullable = "libnccl.so.2" by soname), so the library has no link-time dependency on it; every call below returns
