@@ -170,7 +170,7 @@ def check(code: int, what: str) -> None:
 
 
 # kernels launched per ABI call (bench.py reports the total as gpu_launches)
-KERNELS_PER_CALL = {"ctx_mlp_bwd": 3, "ctx_mlp_wgrad": 2, "ctx_mlp_wgrad_ex": 2, "ctx_composite_train": 2, "ctx_composite_train_noise": 2, "ctx_render_rays": 6, "ctx_render_rays_ndc": 6, "ctx_image_metrics": 2, "ctx_allreduce": 0, "ctx_comm_load": 0, "ctx_comm_unique_id": 0, "ctx_comm_init": 0, "ctx_comm_destroy": 0}     # (the view-direction wgrad also runs a small post kernel: +1, counted by the callers that know the net)
+KERNELS_PER_CALL = {"ctx_mlp_bwd": 3, "ctx_mlp_wgrad": 2, "ctx_mlp_wgrad_ex": 2, "ctx_composite_train": 2, "ctx_composite_train_noise": 2, "ctx_render_rays": 6, "ctx_render_rays_ndc": 6, "ctx_image_metrics": 2, "ctx_allreduce": 0, "ctx_comm_load": 0, "ctx_comm_unique_id": 0, "ctx_comm_init": 0, "ctx_comm_destroy": 0}     # (the view-direction wgrad also runs a small post kernel: +1, counted by mlp_bwd.launch_wgrad only)
 launch_count = 0
 
 

@@ -1,5 +1,6 @@
 """Host side of the tcgen05 coordinate MLP: network description, weight
-packing and the autograd Function around ctx_mlp_fwd / ctx_mlp_bwd.
+packing, the forward launcher (ctx_mlp_fwd_ex) and the autograd Function that
+pairs it with the backward of mlp_bwd.py.
 
 The modules keep the reference's parameter names and order
 (/root/reference/src/run_nerf_helpers.py:81-97; trainer.py:888 indexes
@@ -42,6 +43,18 @@ class NetDesc:
     def p(self):
         return ctypes.cast(self.blob, ctypes.c_void_p)
 
+    def record_bytes(self, P: int) -> int:
+        """Bytes of the activation records of P points (the dZ records take as many)."""
+        ntiles = 4 * ((P + 4 * TILE - 1) // (4 * TILE))     # the 2-CTA kernels work on 4 tiles at a time
+        return ntiles * self.act_tile_bytes
+
+    def weight_buffers(self, dev):
+        """Uninitialised (w, wt, fparams) buffers that ctx_mlp_pack fills: the bf16 forward and transposed weight
+        streams and the fp32 bias/head block."""
+        return (torch.empty(self.w_bytes, dtype=torch.uint8, device=dev),
+                torch.empty(max(self.wt_bytes, 16), dtype=torch.uint8, device=dev),
+                torch.empty(self.n_fparams, dtype=torch.float32, device=dev))
+
 
 class PackedWeights:
     """bf16 weight streams (forward + transposed) and the fp32 bias/head block, per device.
@@ -72,15 +85,12 @@ class PackedWeights:
             if (len(refs) == len(params) and all(r() is p for r, p in zip(refs, params))
                     and versions == tuple(p._version for p in params)):
                 return bufs
-        d = self.desc
         for p in params:
             if p.dtype != torch.float32 or not p.is_contiguous() or p.device != dev or not p.is_cuda:
                 raise _lib.CtxNerfError("MLP parameters must be contiguous fp32 tensors on one CUDA device "
                                         "(ctxnerf has no CPU path)")
-        bufs = (torch.empty(d.w_bytes, dtype=torch.uint8, device=dev),
-                torch.empty(max(d.wt_bytes, 16), dtype=torch.uint8, device=dev),
-                torch.empty(d.n_fparams, dtype=torch.float32, device=dev))
-        pack_into(d, params, bufs)
+        bufs = self.desc.weight_buffers(dev)
+        pack_into(self.desc, params, bufs)
         self.generation += 1
         if cacheable:
             self._per_dev[dev] = (tuple(weakref.ref(p) for p in params), tuple(p._version for p in params), bufs)
@@ -96,17 +106,36 @@ def pack_into(desc: NetDesc, params: List[torch.Tensor], bufs):
              ptr(bufs[2]), stream_ptr(dev))
 
 
-def _launch_fwd(desc: NetDesc, w, f, *, x=None, rays=None, P: int, out, acts=None, L_pts=10, L_dirs=4):
-    dev = out.device
-    fn = "ctx_mlp_fwd"
+def launch_fwd(net, packed, out, *, x=None, rays=None, res=None, gather=None, acts=None):
+    """The fused forward of ``net`` with the packed weights ``packed`` = (w, wt, fparams), on the current stream:
+    ``out`` [P, out_ch] receives the raw output and ``acts`` (optional, ``record_bytes(P)`` bytes) the activation
+    records of the backward.  The input picks the kernel's mode:
+
+    * ``x`` [P, in_ch]: encoded inputs (mode 0);
+    * ``rays`` = (rays_o, rays_d, viewdirs, z_vals [.., S]): the points o + d z, encoded in the kernel (mode 1);
+    * ``res``: the res x res UV grid of get_texture_map, made and encoded in the kernel (mode 2);
+    * ``x`` [*, 2|3] raw coordinates with ``gather`` [P] int64, the row of x each point reads (mode 3)."""
+    desc, (w, _, f), P, dev = net._desc, packed, out.shape[0], out.device
+    o = d = v = z = None
+    x_ld = S = L_pts = L_dirs = 0
+    if rays is not None:
+        for t in rays:
+            if t is not None and (not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous()):
+                raise _lib.CtxNerfError("fused ray query needs contiguous fp32 CUDA tensors (rays_o, rays_d, viewdirs, "
+                                        "z_vals); cast with .float().contiguous()")
+        o, d, v, z = rays
+        mode, S, L_pts, L_dirs = 1, z.shape[-1], net.L_pts, net.L_dirs
+    elif res is not None:
+        mode, S, L_pts = 2, res, net.L_pts
+    else:
+        if not x.is_cuda:
+            raise _lib.CtxNerfError("ctxnerf MLP runs on CUDA tensors only (no CPU fallback)")
+        x = x.reshape(-1, x.shape[-1]).float().contiguous()
+        x_ld = x.shape[-1]
+        mode, L_pts = (0, 0) if gather is None else (3, net.L_pts)
     with torch.cuda.device(dev):
-        if x is not None:
-            call(fn, desc.p, ptr(w), ptr(f), 0, ptr(x), x.shape[-1], None, None, None, None, 0, 0, 0, P,
-                 ptr(out), ptr(acts), stream_ptr(dev))
-        else:
-            o, d, v, z = rays
-            call(fn, desc.p, ptr(w), ptr(f), 1, None, 0, ptr(o), ptr(d), ptr(v), ptr(z), z.shape[-1],
-                 L_pts, L_dirs, P, ptr(out), ptr(acts), stream_ptr(dev))
+        call("ctx_mlp_fwd_ex", desc.p, ptr(w), ptr(f), mode, ptr(x), x_ld, ptr(o), ptr(d), ptr(v), ptr(z), S, L_pts,
+             L_dirs, P, ptr(out), ptr(acts), ptr(gather), 0, stream_ptr(dev))
 
 
 def forward_raw(module, *, x=None, rays=None, save_acts=False):
@@ -114,25 +143,10 @@ def forward_raw(module, *, x=None, rays=None, save_acts=False):
     module._ensure()
     desc: NetDesc = module._desc
     packed = module._packed.get(module._param_list())
-    w, wt, f = packed
-    if x is not None:
-        if not x.is_cuda:
-            raise _lib.CtxNerfError("ctxnerf MLP runs on CUDA tensors only (no CPU fallback)")
-        x = x.reshape(-1, x.shape[-1]).float().contiguous()
-        P, dev = x.shape[0], x.device
-    else:
-        for t in rays:
-            if t is not None and (not t.is_cuda or t.dtype != torch.float32 or not t.is_contiguous()):
-                raise _lib.CtxNerfError("fused ray query needs contiguous fp32 CUDA tensors (rays_o, rays_d, viewdirs, "
-                                        "z_vals); cast with .float().contiguous()")
-        z = rays[3]
-        P, dev = z.numel(), z.device
+    P, dev = (x.shape[:-1].numel(), x.device) if x is not None else (rays[3].numel(), rays[3].device)
     out = torch.empty(P, desc.out_ch, device=dev, dtype=torch.float32)
-    acts = None
-    if save_acts:
-        ntiles = 4 * ((P + 4 * TILE - 1) // (4 * TILE))     # the 2-CTA kernels work on 4 tiles at a time
-        acts = torch.empty(ntiles * desc.act_tile_bytes, dtype=torch.uint8, device=dev)
-    _launch_fwd(desc, w, f, x=x, rays=rays, P=P, out=out, acts=acts, L_pts=module.L_pts, L_dirs=module.L_dirs)
+    acts = torch.empty(desc.record_bytes(P), dtype=torch.uint8, device=dev) if save_acts else None
+    launch_fwd(module, packed, out, x=x, rays=rays, acts=acts)
     return out, acts, P, packed
 
 

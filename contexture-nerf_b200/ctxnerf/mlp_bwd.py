@@ -1,72 +1,64 @@
-"""Host side of the MLP backward: allocates the gradient tensors and the dZ
-scratch records and calls ctx_mlp_bwd (dgrad + wgrad kernels)."""
+"""Host side of the MLP backward: the dgrad (ctx_mlp_dgrad_ex) and wgrad (ctx_mlp_wgrad_ex) launchers, which write
+into buffers the caller owns, and the functions that allocate those buffers for one backward pass."""
 from __future__ import annotations
 
 import ctypes
 
 import torch
 
+from . import _lib
 from ._lib import call, ptr, stream_ptr
 
 
-def _grad_targets(module, sinks, dev):
-    params = module._param_list()
-    if sinks is not None:
-        return sinks, params
-    sizes = [p.numel() for p in params]
-    flat = torch.zeros(sum(sizes), device=dev, dtype=torch.float32)
-    grads, off = [], 0
-    for p, n in zip(params, sizes):
-        grads.append(flat[off:off + n].view_as(p))
-        off += n
-    return grads, params
-
-
-def mlp_dgrad(module, packed, acts, P, g_out, max_sms=0):
-    """dZ records of every GEMM layer from g_out (ctx_mlp_dgrad_ex).  ``max_sms`` > 0 limits the SMs the kernel
-    occupies so that another kernel can run beside it."""
-    desc = module._desc
+def launch_dgrad(net, packed, g_out, acts, dacts, P, max_sms=0):
+    """dZ records ``dacts`` of every GEMM layer from g_out [P, out_ch] (fp32, contiguous) and the activation records
+    ``acts``.  ``max_sms`` > 0 limits the SMs the kernel occupies so that another kernel can run beside it."""
     _, wt, f = packed
     dev = g_out.device
-    g = g_out.reshape(P, desc.out_ch).float().contiguous()
-    dacts = torch.empty_like(acts)
     with torch.cuda.device(dev):
-        call("ctx_mlp_dgrad_ex", desc.p, ptr(wt), ptr(f), ptr(g), ptr(acts), ptr(dacts), P, int(max_sms),
+        call("ctx_mlp_dgrad_ex", net._desc.p, ptr(wt), ptr(f), ptr(g_out), ptr(acts), ptr(dacts), P, int(max_sms),
              stream_ptr(dev))
-    return dacts
+
+
+def launch_wgrad(net, acts, dacts, P, grads, scratch, max_sms=0):
+    """Accumulates (+=) the parameter gradients into ``grads`` (fp32 tensors in ``net._param_list()`` order) from the
+    activation and dZ records; ``scratch`` is ``wgrad_scratch``."""
+    params = net._param_list()
+    garr = (ctypes.c_void_p * len(grads))(*[t.data_ptr() for t in grads])
+    parr = (ctypes.c_void_p * len(params))(*[t.data_ptr() for t in params])
+    if net._desc.in_views > 0:
+        _lib.launch_count += 1     # the view-direction head's post kernel
+    dev = acts.device
+    with torch.cuda.device(dev):
+        call("ctx_mlp_wgrad_ex", net._desc.p, ptr(acts), ptr(dacts), P, ctypes.cast(garr, ctypes.c_void_p), len(grads),
+             ctypes.cast(parr, ctypes.c_void_p), ptr(scratch), int(max_sms), stream_ptr(dev))
 
 
 def wgrad_scratch(dev):
     """fp32 scratch of the wgrad kernels (ctx_mlp_wgrad_scratch_floats floats): the per-CTA partial sums and the
     view-direction head's G job."""
-    from . import _lib
     return torch.empty(_lib.lib().ctx_mlp_wgrad_scratch_floats(), device=dev, dtype=torch.float32)
 
 
-def mlp_wgrad(module, acts, dacts, P, sinks=None, max_sms=0, scratch=None):
-    """Parameter gradients from the activation and dZ records (ctx_mlp_wgrad_ex); accumulates into ``sinks`` when
-    given (returns None), else returns fresh tensors."""
-    dev = acts.device
-    grads, params = _grad_targets(module, sinks, dev)
-    arr = (ctypes.c_void_p * len(grads))(*[t.data_ptr() for t in grads])
-    parr = (ctypes.c_void_p * len(params))(*[t.data_ptr() for t in params])
-    if scratch is None:
-        scratch = wgrad_scratch(dev)
-    with torch.cuda.device(dev):
-        call("ctx_mlp_wgrad_ex", module._desc.p, ptr(acts), ptr(dacts), P, ctypes.cast(arr, ctypes.c_void_p),
-             len(grads), ctypes.cast(parr, ctypes.c_void_p), ptr(scratch), int(max_sms), stream_ptr(dev))
-    if sinks is not None:
-        return None
+def mlp_dgrad(module, packed, acts, P, g_out, max_sms=0):
+    """Fresh dZ records from g_out (``launch_dgrad``)."""
+    g = g_out.reshape(P, module._desc.out_ch).float().contiguous()
+    dacts = torch.empty_like(acts)
+    launch_dgrad(module, packed, g, acts, dacts, P, max_sms)
+    return dacts
+
+
+def mlp_wgrad(module, acts, dacts, P, max_sms=0):
+    """Fresh parameter gradients from the activation and dZ records (``launch_wgrad``): one tensor per parameter,
+    None for a parameter that does not require a gradient."""
+    params = module._param_list()
+    sizes = [p.numel() for p in params]
+    flat = torch.zeros(sum(sizes), device=acts.device, dtype=torch.float32)
+    grads = [t.view_as(p) for t, p in zip(flat.split(sizes), params)]
+    launch_wgrad(module, acts, dacts, P, grads, wgrad_scratch(acts.device), max_sms)
     return [gr if p.requires_grad else None for gr, p in zip(grads, params)]
 
 
-def mlp_backward(module, packed, acts, P, g_out, sinks=None, timed=None):
-    """Gradients w.r.t. the module's parameters: dgrad then wgrad on the current stream.
-
-    ``sinks`` (list of fp32 tensors, one per parameter, e.g. views into a flat
-    all-reduce bucket): the wgrad kernel accumulates straight into them and
-    ``None`` is returned; otherwise fresh zeroed tensors are returned.
-    ``timed(name, fn)`` (optional) wraps the two kernel launches ("dgrad", "wgrad")."""
-    run = timed if timed is not None else (lambda name, fn: fn())
-    dacts = run("dgrad", lambda: mlp_dgrad(module, packed, acts, P, g_out))
-    return run("wgrad", lambda: mlp_wgrad(module, acts, dacts, P, sinks))
+def mlp_backward(module, packed, acts, P, g_out):
+    """Gradients w.r.t. the module's parameters: dgrad then wgrad on the current stream."""
+    return mlp_wgrad(module, acts, mlp_dgrad(module, packed, acts, P, g_out), P)

@@ -15,7 +15,7 @@ import torch
 
 from . import _lib
 from ._lib import call, ptr, stream_ptr
-from .mlp import TILE
+from .mlp import launch_fwd
 from .mlp_bwd import mlp_backward
 
 
@@ -29,16 +29,11 @@ class _TextureMapFn(torch.autograd.Function):
         dev = params[0].device
         P = res * res
         packed = module._packed.get(list(params))
-        w, wt, f = packed
         raw = torch.empty(P, desc.out_ch, device=dev, dtype=torch.float32)
-        acts = None
-        if need_grad:
-            ntiles = 4 * ((P + 4 * TILE - 1) // (4 * TILE))
-            acts = torch.empty(ntiles * desc.act_tile_bytes, dtype=torch.uint8, device=dev)
+        acts = torch.empty(desc.record_bytes(P), dtype=torch.uint8, device=dev) if need_grad else None
         tex = torch.empty(1, desc.out_ch, res, res, device=dev, dtype=torch.float32)
+        launch_fwd(module, packed, raw, res=res, acts=acts)
         with torch.cuda.device(dev):
-            call("ctx_mlp_fwd", desc.p, ptr(w), ptr(f), 2, None, 0, None, None, None, None, res, module.L_pts, 0, P,
-                 ptr(raw), ptr(acts), stream_ptr(dev))
             call("ctx_tanh01_fwd", ptr(raw), ptr(tex), P, desc.out_ch, stream_ptr(dev))
         ctx.module, ctx.P, ctx.acts, ctx.packed, ctx.raw = module, P, acts, packed, raw
         return tex, raw
@@ -83,16 +78,11 @@ class _TextureValidFn(torch.autograd.Function):
         dev = params[0].device
         M = idx.numel()
         packed = module._packed.get(list(params))
-        w, wt, f = packed
         raw = torch.empty(M, desc.out_ch, device=dev, dtype=torch.float32)
-        acts = None
-        if need_grad and M:
-            ntiles = 4 * ((M + 4 * TILE - 1) // (4 * TILE))
-            acts = torch.empty(ntiles * desc.act_tile_bytes, dtype=torch.uint8, device=dev)
+        acts = torch.empty(desc.record_bytes(M), dtype=torch.uint8, device=dev) if need_grad and M else None
         final = torch.empty(n_pix, desc.out_ch, device=dev, dtype=torch.float32)
+        launch_fwd(module, packed, raw, x=uvs, gather=idx, acts=acts)
         with torch.cuda.device(dev):
-            call("ctx_mlp_fwd_ex", desc.p, ptr(w), ptr(f), 3, ptr(uvs), 2, None, None, None, None, 1, module.L_pts, 0, M,
-                 ptr(raw), ptr(acts), ptr(idx), 0, stream_ptr(dev))
             call("ctx_rows_scatter", ptr(raw), ptr(idx), float(scale), ptr(final), M, n_pix, desc.out_ch, stream_ptr(dev))
         ctx.module, ctx.M, ctx.acts, ctx.packed, ctx.idx, ctx.scale = module, M, acts, packed, idx, float(scale)
         return final

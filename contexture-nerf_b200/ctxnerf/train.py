@@ -26,8 +26,8 @@ import torch
 from . import _lib, ops
 from ._lib import CtxNerfError, call, ptr, stream_ptr
 from .dist import BucketComm, FlatBucket, dist_backend, world
-from .mlp import TILE, forward_raw, pack_into
-from .mlp_bwd import wgrad_scratch
+from .mlp import launch_fwd, pack_into
+from .mlp_bwd import launch_dgrad, launch_wgrad, wgrad_scratch
 from .run_nerf_helpers import NeRF
 
 
@@ -56,8 +56,7 @@ class _Plan:
         self.rgb0, self.rgb = torch.empty(R, 3, **f32), torch.empty(R, 3, **f32)
 
         def records(P, net):
-            ntiles = 4 * ((P + 4 * TILE - 1) // (4 * TILE))     # the 2-CTA kernels work on 4 tiles at a time
-            n = ntiles * net._desc.act_tile_bytes
+            n = net._desc.record_bytes(P)
             return (torch.empty(n, dtype=torch.uint8, device=dev), torch.empty(n, dtype=torch.uint8, device=dev))
 
         self.acts_c, self.dacts_c = records(R * S, tr.coarse)
@@ -175,12 +174,7 @@ class NerfTrainer:
             im = im.to(dev).float().div_(255.0) if im.dtype == torch.uint8 else im.to(dev, dtype=torch.float32)
             self.images = im.contiguous()
         # bf16 weight streams of both networks: trainer-owned static buffers, re-packed after every Adam update
-        self._pk = {}
-        for net in (self.coarse, self.fine):
-            d = net._desc
-            self._pk[net] = (torch.empty(d.w_bytes, dtype=torch.uint8, device=dev),
-                             torch.empty(max(d.wt_bytes, 16), dtype=torch.uint8, device=dev),
-                             torch.empty(d.n_fparams, dtype=torch.float32, device=dev))
+        self._pk = {net: net._desc.weight_buffers(dev) for net in (self.coarse, self.fine)}
         self._scratch = {net: wgrad_scratch(dev) for net in (self.coarse, self.fine)}
         self._packed_version = -1
         self._plans = {}
@@ -248,33 +242,12 @@ class NerfTrainer:
         pack_into(self.coarse._desc, self.coarse._param_list(), self._pk[self.coarse])
         main.wait_event(self._ev3)
 
-    def _fwd(self, net, rays, P, out, acts):
-        o, d, v, z = rays
-        w, _, f = self._pk[net]
-        call("ctx_mlp_fwd_ex", net._desc.p, ptr(w), ptr(f), 1, None, 0, ptr(o), ptr(d), ptr(v), ptr(z), z.shape[-1],
-             net.L_pts, net.L_dirs, P, ptr(out), ptr(acts), None, 0, stream_ptr(self.device))
-
-    def _dgrad(self, net, g_raw, acts, dacts, P, max_sms=0):
-        _, wt, f = self._pk[net]
-        call("ctx_mlp_dgrad_ex", net._desc.p, ptr(wt), ptr(f), ptr(g_raw), ptr(acts), ptr(dacts), P, int(max_sms),
-             stream_ptr(self.device))
-
-    def _wgrad(self, net, acts, dacts, P, max_sms=0):
-        sinks, params = self.bucket.sinks_for(net), net._param_list()
-        garr = (ctypes.c_void_p * len(sinks))(*[t.data_ptr() for t in sinks])
-        parr = (ctypes.c_void_p * len(params))(*[t.data_ptr() for t in params])
-        _lib.launch_count += 1     # the view-direction head's post kernel
-        call("ctx_mlp_wgrad_ex", net._desc.p, ptr(acts), ptr(dacts), P, ctypes.cast(garr, ctypes.c_void_p), len(sinks),
-             ctypes.cast(parr, ctypes.c_void_p), ptr(self._scratch[net]), int(max_sms), stream_ptr(self.device))
-
     def _comp_train(self, raw, z, d, R, S, target, g_raw, weights, rgb, noise_stream):
-        if self.raw_noise_std > 0.0:     # the raygen key (seed0 + counter), its own Philox stream per pass
-            call("ctx_composite_train_noise", ptr(raw), ptr(z), ptr(d), R, S, int(self.white_bkgd), ptr(target),
-                 1.0 / (3.0 * R), ptr(self._loss), ptr(g_raw), ptr(weights), ptr(rgb), self.raw_noise_std,
-                 self._seed0, ptr(self._ctr), noise_stream, stream_ptr(self.device))
-            return
-        call("ctx_composite_train", ptr(raw), ptr(z), ptr(d), None, R, S, int(self.white_bkgd), ptr(target),
-             1.0 / (3.0 * R), ptr(self._loss), ptr(g_raw), ptr(weights), ptr(rgb), stream_ptr(self.device))
+        # the noise has the raygen key (seed0 + counter) and its own Philox stream per pass; raw_noise_std == 0 runs
+        # the launches of ctx_composite_train without noise
+        call("ctx_composite_train_noise", ptr(raw), ptr(z), ptr(d), R, S, int(self.white_bkgd), ptr(target),
+             1.0 / (3.0 * R), ptr(self._loss), ptr(g_raw), ptr(weights), ptr(rgb), self.raw_noise_std,
+             self._seed0, ptr(self._ctr), noise_stream, stream_ptr(self.device))
 
     # --------------------------------------------------------- the step body
     def _enqueue_head(self, pl: _Plan):
@@ -294,20 +267,27 @@ class NerfTrainer:
         ops.raygen(self.H, self.W, self.K, self.c2w if self.n_views == 1 else self.poses, ray_idx=pl.idx, n_samples=S,
                    near=self.near, far=self.far, lindisp=self.lindisp, perturb=jit, seed=self._seed0, seed_dev=self._ctr if jit else None,
                    ndc=self._ndc_args(self.K), want_viewdirs=True, out=(pl.o, pl.d, pl.v, pl.z_c))
-        rays_c, rays_f = (pl.o, pl.d, pl.v, pl.z_c), (pl.o, pl.d, pl.v, pl.z_f)
-        self._timed("mlp_fwd_coarse", lambda: self._fwd(self.coarse, rays_c, Pc, pl.raw_c, pl.acts_c))
+        c, f, pk, sinks = self.coarse, self.fine, self._pk, self.bucket.sinks_for
+        self._timed("mlp_fwd_coarse", lambda: launch_fwd(c, pk[c], pl.raw_c, rays=(pl.o, pl.d, pl.v, pl.z_c),
+                                                         acts=pl.acts_c))
         # raw2outputs + img2mse(rgb0, target) + their backward in one pass; the weights feed sample_pdf
         self._comp_train(pl.raw_c, pl.z_c, pl.d, R, S, pl.target, pl.g_raw_c, pl.w_c, pl.rgb0, 2)
         ops.resample_merge(pl.z_c, pl.w_c, Ni, det=not jit, seed=self._seed0 + 1, seed_dev=self._ctr if jit else None,
                            out=(pl.zs, pl.z_f))
-        self._timed("mlp_fwd_fine", lambda: self._fwd(self.fine, rays_f, Pf, pl.raw_f, pl.acts_f))
+        self._timed("mlp_fwd_fine", lambda: launch_fwd(f, pk[f], pl.raw_f, rays=(pl.o, pl.d, pl.v, pl.z_f),
+                                                       acts=pl.acts_f))
         self._comp_train(pl.raw_f, pl.z_f, pl.d, R, Sf, pl.target, pl.g_raw_f, None, pl.rgb, 3)
-        self._timed("mlp_dgrad_fine", lambda: self._dgrad(self.fine, pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf))
+        self._timed("mlp_dgrad_fine", lambda: launch_dgrad(f, pk[f], pl.g_raw_f, pl.acts_f, pl.dacts_f, Pf))
 
         def coarse_chain(dgrad_sms):
             self._timed("mlp_dgrad_coarse",
-                        lambda: self._dgrad(self.coarse, pl.g_raw_c, pl.acts_c, pl.dacts_c, Pc, max_sms=dgrad_sms))
-            self._timed("mlp_wgrad_coarse", lambda: self._wgrad(self.coarse, pl.acts_c, pl.dacts_c, Pc))
+                        lambda: launch_dgrad(c, pk[c], pl.g_raw_c, pl.acts_c, pl.dacts_c, Pc, dgrad_sms))
+            self._timed("mlp_wgrad_coarse",
+                        lambda: launch_wgrad(c, pl.acts_c, pl.dacts_c, Pc, sinks(c), self._scratch[c]))
+
+        def wgrad_fine(max_sms):
+            self._timed("mlp_wgrad_fine",
+                        lambda: launch_wgrad(f, pl.acts_f, pl.dacts_f, Pf, sinks(f), self._scratch[f], max_sms))
 
         if self.overlap_backward:
             self._ev0.record(main)
@@ -318,15 +298,14 @@ class NerfTrainer:
             with torch.cuda.stream(self._side):
                 coarse_chain(self.side_sms)
                 self._ev1.record(self._side)
-            self._timed("mlp_wgrad_fine", lambda: self._wgrad(self.fine, pl.acts_f, pl.dacts_f, Pf,
-                                                              max_sms=self.n_sms - self.side_sms))
+            wgrad_fine(self.n_sms - self.side_sms)
             main.wait_event(self._ev1)
             if self.timers is not None:   # span of the concurrent group on the main stream
                 g1 = torch.cuda.Event(enable_timing=True)
                 g1.record(main)
                 self.timers.setdefault("bwd_overlap_group", []).append((g0, g1))
         else:
-            self._timed("mlp_wgrad_fine", lambda: self._wgrad(self.fine, pl.acts_f, pl.dacts_f, Pf))
+            wgrad_fine(0)
             coarse_chain(0)
 
     def _enqueue_tail(self):
@@ -353,12 +332,35 @@ class NerfTrainer:
         """(focal, near) of the NDC warp upstream applies to forward-facing scenes, or None"""
         return (float(K[0][0]), 1.0) if self.ndc else None
 
-    def _call_render(self, a, K):
+    def _render_rays(self, H, W, K, pose, ray_idx, n_rays, near, far, nets, bufs, n_samples, n_importance=0,
+                     lindisp=False, perturb=False, seed=0, sphere=None):
+        """One ctx_render_rays (ctx_render_rays_ndc on an NDC trainer) of ``n_rays`` > 0 rays of the device pose
+        ``pose``: ``nets`` holds the network of the first pass and, with ``n_importance`` > 0, the fine one; ``bufs``
+        maps CtxRenderArgs buffer fields to device tensors (the others stay NULL); ``sphere``: (cx, cy, cz, r)."""
+        a = _lib.CtxRenderArgs()
+        a.H, a.W = int(H), int(W)
+        a.fx, a.fy, a.cx, a.cy = float(K[0][0]), float(K[1][1]), float(K[0][2]), float(K[1][2])
+        a.c2w, a.c2w_ld = pose.data_ptr(), pose.stride(0)
+        a.ray_idx, a.n_rays = (None if ray_idx is None else ray_idx.data_ptr()), n_rays
+        a.near, a.far, a.lindisp, a.perturb = float(near), float(far), int(lindisp), int(bool(perturb))
+        a.seed = int(seed)
+        sph = None      # the sphere array must outlive the call
+        if sphere is not None:
+            sph = (ctypes.c_float * 4)(*[float(x) for x in sphere])
+            a.sphere = ctypes.addressof(sph)
+        a.n_samples, a.n_importance, a.white_bkgd = int(n_samples), int(n_importance), int(self.white_bkgd)
+        a.L_pts, a.L_dirs = nets[0].L_pts, nets[0].L_dirs
+        for cn, net in zip((a.coarse, a.fine), nets):
+            w, _, f = self._pk[net]
+            cn.desc, cn.wpacked, cn.fparams = ctypes.addressof(net._desc.blob), w.data_ptr(), f.data_ptr()
+        for name, t in bufs.items():
+            setattr(a, name, t.data_ptr())
         nd = self._ndc_args(K)
-        if nd is None:
-            call("ctx_render_rays", ctypes.byref(a), stream_ptr(self.device))
-        else:
-            call("ctx_render_rays_ndc", ctypes.byref(a), nd[0], nd[1], stream_ptr(self.device))
+        with torch.cuda.device(self.device):
+            if nd is None:
+                call("ctx_render_rays", ctypes.byref(a), stream_ptr(self.device))
+            else:
+                call("ctx_render_rays_ndc", ctypes.byref(a), nd[0], nd[1], stream_ptr(self.device))
 
     # ------------------------------------------------------------------- API
     @torch.no_grad()
@@ -485,7 +487,7 @@ class NerfTrainer:
         return done     # loss_pinned is valid once this event has completed
 
     # ------------------------------------------------------------ inference
-    def _render(self, ray_idx, perturb, seed=0, max_sms=0, c2w=None):
+    def _render(self, ray_idx, perturb, seed=0, c2w=None):
         """Forward-only coarse+fine render of the given pixels (None = the whole image): dynamic shapes, fresh
         outputs; shares the trainer's packed weights.  ONE C-ABI call: ctx_render_rays (csrc/render.cu) enqueues
         raygen -> MLP -> raw2outputs -> sample_pdf + merge -> MLP -> raw2outputs."""
@@ -494,53 +496,23 @@ class NerfTrainer:
             ray_idx = ray_idx.to(device=dev, dtype=torch.int64).reshape(-1).contiguous()
         R = self.H * self.W if ray_idx is None else ray_idx.numel()
         f32 = dict(device=dev, dtype=torch.float32)
-        o, d, v = (torch.empty(R, 3, **f32) for _ in range(3))
-        z_c, raw_c, w_c = torch.empty(R, S, **f32), torch.empty(R * S, 4, **f32), torch.empty(R, S, **f32)
-        zs, z_f = torch.empty(R, Ni, **f32), torch.empty(R, S + Ni, **f32)
-        raw_f, w_f = torch.empty(R * (S + Ni), 4, **f32), torch.empty(R, S + Ni, **f32)
-        maps_c = [torch.empty(R, 3, **f32)] + [torch.empty(R, **f32) for _ in range(3)]     # rgb, disp, acc, depth
-        maps_f = [torch.empty(R, 3, **f32)] + [torch.empty(R, **f32) for _ in range(3)]
-        if R == 0:
-            return dict(comp_c=(maps_c[0], maps_c[1], maps_c[2], w_c, maps_c[3]),
-                        comp_f=(maps_f[0], maps_f[1], maps_f[2], w_f, maps_f[3]), z_f=z_f, raw_f=raw_f, R=0)
-        a = _lib.CtxRenderArgs()
-        a.H, a.W = self.H, self.W
-        a.fx, a.fy, a.cx, a.cy = (float(self.K[0][0]), float(self.K[1][1]), float(self.K[0][2]), float(self.K[1][2]))
-        pose = self.c2w
-        if c2w is not None:
-            pose = torch.as_tensor(c2w, dtype=torch.float32).to(dev).contiguous()
-            if tuple(pose.shape) not in ((3, 4), (4, 4)):
-                raise CtxNerfError(f"NerfTrainer.render: c2w must be one pose [3|4, 4], got {tuple(pose.shape)}")
-        a.c2w, a.c2w_ld = pose.data_ptr(), pose.stride(0)
-        a.ray_idx, a.n_rays = (None if ray_idx is None else ray_idx.data_ptr()), R
-        a.near, a.far, a.lindisp, a.perturb = self.near, self.far, int(self.lindisp), int(bool(perturb))
-        a.seed, a.seed_dev, a.sphere = int(seed), None, None
-        a.n_samples, a.n_importance, a.white_bkgd = S, Ni, int(self.white_bkgd)
-        a.L_pts, a.L_dirs, a.max_sms = self.coarse.L_pts, self.coarse.L_dirs, int(max_sms)
-        for field, net in (("coarse", self.coarse), ("fine", self.fine)):
-            w, _, f = self._pk[net]
-            cn = getattr(a, field)
-            cn.desc, cn.wpacked, cn.fparams = ctypes.addressof(net._desc.blob), w.data_ptr(), f.data_ptr()
-        for name, t in (("rays_o", o), ("rays_d", d), ("viewdirs", v), ("z_coarse", z_c), ("raw_coarse", raw_c),
-                        ("weights_coarse", w_c), ("z_samples", zs), ("z_fine", z_f), ("raw_fine", raw_f),
-                        ("weights_fine", w_f), ("rgb0", maps_c[0]), ("disp0", maps_c[1]), ("acc0", maps_c[2]),
-                        ("depth0", maps_c[3]), ("rgb_map", maps_f[0]), ("disp_map", maps_f[1]), ("acc_map", maps_f[2]),
-                        ("depth_map", maps_f[3])):
-            setattr(a, name, t.data_ptr())
-        self._call_render(a, self.K)
-        return dict(comp_c=(maps_c[0], maps_c[1], maps_c[2], w_c, maps_c[3]),
-                    comp_f=(maps_f[0], maps_f[1], maps_f[2], w_f, maps_f[3]), z_f=z_f, raw_f=raw_f, R=R)
-
-    def _composite(self, raw, z, d, R, S):
-        dev = self.device
-        rgb = torch.empty(R, 3, device=dev)
-        disp = torch.empty(R, device=dev)
-        acc = torch.empty(R, device=dev)
-        w = torch.empty(R, S, device=dev)
-        depth = torch.empty(R, device=dev)
-        call("ctx_composite_fwd", ptr(raw), ptr(z), ptr(d), None, R, S, int(self.white_bkgd), ptr(rgb), ptr(disp),
-             ptr(acc), ptr(w), ptr(depth), stream_ptr(dev))
-        return rgb, disp, acc, w, depth
+        b = {n: torch.empty(R, 3, **f32) for n in ("rays_o", "rays_d", "viewdirs", "rgb0", "rgb_map")}
+        b.update({n: torch.empty(R, **f32) for n in ("disp0", "acc0", "depth0", "disp_map", "acc_map", "depth_map")})
+        b.update({n: torch.empty(R, S, **f32) for n in ("z_coarse", "weights_coarse")})
+        b.update({n: torch.empty(R, S + Ni, **f32) for n in ("z_fine", "weights_fine")})
+        b.update(raw_coarse=torch.empty(R * S, 4, **f32), z_samples=torch.empty(R, Ni, **f32),
+                 raw_fine=torch.empty(R * (S + Ni), 4, **f32))
+        if R > 0:
+            pose = self.c2w
+            if c2w is not None:
+                pose = torch.as_tensor(c2w, dtype=torch.float32).to(dev).contiguous()
+                if tuple(pose.shape) not in ((3, 4), (4, 4)):
+                    raise CtxNerfError(f"NerfTrainer.render: c2w must be one pose [3|4, 4], got {tuple(pose.shape)}")
+            self._render_rays(self.H, self.W, self.K, pose, ray_idx, R, self.near, self.far, (self.coarse, self.fine),
+                              b, S, Ni, lindisp=self.lindisp, perturb=perturb, seed=seed)
+        return dict(comp_c=tuple(b[n] for n in ("rgb0", "disp0", "acc0", "weights_coarse", "depth0")),
+                    comp_f=tuple(b[n] for n in ("rgb_map", "disp_map", "acc_map", "weights_fine", "depth_map")),
+                    z_f=b["z_fine"], raw_f=b["raw_fine"], R=R)
 
     @torch.no_grad()
     def render(self, ray_idx: Optional[torch.Tensor] = None, c2w=None):
@@ -613,32 +585,15 @@ class NerfTrainer:
         if ray_idx is not None:
             ray_idx = ray_idx.to(device=dev, dtype=torch.int64).reshape(-1).contiguous()
         n = H * W if ray_idx is None else ray_idx.numel()
-        o, d, v = (torch.empty(n, 3, **f32) for _ in range(3))
-        z, raw, w = torch.empty(n, n_samples, **f32), torch.empty(n * n_samples, 4, **f32), torch.empty(n, n_samples, **f32)
-        rgb, disp, acc, depth = torch.empty(n, 3, **f32), torch.empty(n, **f32), torch.empty(n, **f32), torch.empty(n, **f32)
+        b = {k: torch.empty(n, 3, **f32) for k in ("rays_o", "rays_d", "viewdirs", "rgb_map")}
+        b.update({k: torch.empty(n, **f32) for k in ("disp_map", "acc_map", "depth_map")})
+        b.update({k: torch.empty(n, n_samples, **f32) for k in ("z_coarse", "weights_coarse")})
+        b.update(raw_coarse=torch.empty(n * n_samples, 4, **f32))
         if n > 0:
             # the single-pass form of ctx_render_rays (n_importance = 0) with the fine network and the sphere interval
-            a = _lib.CtxRenderArgs()
-            a.H, a.W = int(H), int(W)
-            a.fx, a.fy, a.cx, a.cy = float(K[0][0]), float(K[1][1]), float(K[0][2]), float(K[1][2])
-            a.c2w, a.c2w_ld = c2w_d.data_ptr(), c2w_d.stride(0)
-            a.ray_idx, a.n_rays = (None if ray_idx is None else ray_idx.data_ptr()), n
-            a.near, a.far = float(self.near if near is None else near), float(self.far if far is None else far)
-            a.lindisp, a.perturb, a.seed, a.seed_dev = 0, 0, 0, None
-            sph = None
-            if sphere is not None:
-                sph = (ctypes.c_float * 4)(*[float(x) for x in sphere])
-                a.sphere = ctypes.addressof(sph)
-            a.n_samples, a.n_importance, a.white_bkgd = int(n_samples), 0, int(self.white_bkgd)
-            a.L_pts, a.L_dirs, a.max_sms = self.fine.L_pts, self.fine.L_dirs, 0
-            wp, _, fp = self._pk[self.fine]
-            a.coarse.desc, a.coarse.wpacked, a.coarse.fparams = ctypes.addressof(self.fine._desc.blob), wp.data_ptr(), fp.data_ptr()
-            for name, t in (("rays_o", o), ("rays_d", d), ("viewdirs", v), ("z_coarse", z), ("raw_coarse", raw),
-                            ("weights_coarse", w), ("rgb_map", rgb), ("disp_map", disp), ("acc_map", acc),
-                            ("depth_map", depth)):
-                setattr(a, name, t.data_ptr())
-            with torch.cuda.device(dev):
-                self._call_render(a, K)
+            self._render_rays(H, W, K, c2w_d, ray_idx, n, self.near if near is None else near,
+                              self.far if far is None else far, (self.fine,), b, n_samples, sphere=sphere)
+        rgb, disp, acc, depth = b["rgb_map"], b["disp_map"], b["acc_map"], b["depth_map"]
         if ray_idx is None:
             return dict(rgb_map=rgb.reshape(H, W, 3), disp_map=disp.reshape(H, W), acc_map=acc.reshape(H, W),
                         depth_map=depth.reshape(H, W))

@@ -324,6 +324,7 @@ def test_ndc_render_equals_the_kernel_sequence(cuda):
     for bit; ctx_render_rays without NDC is unchanged; the metric sphere interval is refused."""
     from ctxnerf import _lib, ops
     from ctxnerf._lib import CtxNerfError
+    from ctxnerf.mlp import launch_fwd
     tr, K, c2w = _trainer(cuda, 48, 64, 50.0, N_importance=128)
     flat, _, _ = _trainer(cuda, 48, 64, 50.0, N_importance=128, ndc=False, near=0.5, far=4.0)
     idx = torch.randint(0, 48 * 64, (1500,), device=cuda)
@@ -334,12 +335,12 @@ def test_ndc_render_equals_the_kernel_sequence(cuda):
                        want_viewdirs=True)
         o, d, v, z_c = r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]
         raw_c = torch.empty(1500 * S, 4, device=cuda)
-        t._fwd(t.coarse, (o, d, v, z_c), 1500 * S, raw_c, None)
-        comp_c = t._composite(raw_c, z_c, d, 1500, S)
+        launch_fwd(t.coarse, t._pk[t.coarse], raw_c, rays=(o, d, v, z_c))
+        comp_c = ops.composite(raw_c.view(1500, S, 4), z_c, d, white_bkgd=t.white_bkgd)
         zs, z_f = ops.resample_merge(z_c, comp_c[3], Ni, det=True, seed=1)
         raw_f = torch.empty(1500 * (S + Ni), 4, device=cuda)
-        t._fwd(t.fine, (o, d, v, z_f), 1500 * (S + Ni), raw_f, None)
-        rgb, disp, acc, _, depth = t._composite(raw_f, z_f, d, 1500, S + Ni)
+        launch_fwd(t.fine, t._pk[t.fine], raw_f, rays=(o, d, v, z_f))
+        rgb, disp, acc, _, depth = ops.composite(raw_f.view(1500, S + Ni, 4), z_f, d, white_bkgd=t.white_bkgd)
         torch.cuda.synchronize()
         assert torch.equal(got["rgb_map"], rgb) and torch.equal(got["acc_map"], acc)
         assert torch.equal(got["depth_map"], depth) and torch.equal(got["rgb0"], comp_c[0])
@@ -353,8 +354,8 @@ def test_ndc_render_equals_the_kernel_sequence(cuda):
     r = ops.raygen(40, 40, Kv, cv.to(cuda), ray_idx=idx2, n_samples=96, near=0.0, far=1.0, ndc=(35.0, 1.0),
                    want_viewdirs=True)
     raw = torch.empty(700 * 96, 4, device=cuda)
-    tr._fwd(tr.fine, (r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]), 700 * 96, raw, None)
-    rgb, _, acc, _, _ = tr._composite(raw, r["z_vals"], r["rays_d"], 700, 96)
+    launch_fwd(tr.fine, tr._pk[tr.fine], raw, rays=(r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]))
+    rgb, _, acc, _, _ = ops.composite(raw.view(700, 96, 4), r["z_vals"], r["rays_d"], white_bkgd=tr.white_bkgd)
     torch.cuda.synchronize()
     assert torch.equal(got["rgb_map"], rgb) and torch.equal(got["acc_map"], acc)
     with pytest.raises(CtxNerfError):

@@ -334,6 +334,7 @@ def test_a_single_pose_stack_changes_nothing(cuda, monkeypatch):
 # ---------------------------------------------------------------- 7. render(c2w=...)
 def test_render_of_a_pose_equals_the_kernel_sequence(cuda):
     from ctxnerf import ops
+    from ctxnerf.mlp import launch_fwd
     for ndc in (True, False):
         tr, K, poses = _mv_trainer(cuda, 3, 48, 64, 50.0, N_importance=128, ndc=ndc,
                                    **({} if ndc else dict(near=0.5, far=4.0)))
@@ -348,12 +349,12 @@ def test_render_of_a_pose_equals_the_kernel_sequence(cuda):
                            want_viewdirs=True)
             o, d, v, z_c = r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]
             raw_c = torch.empty(1500 * S, 4, device=cuda)
-            tr._fwd(tr.coarse, (o, d, v, z_c), 1500 * S, raw_c, None)
-            comp_c = tr._composite(raw_c, z_c, d, 1500, S)
+            launch_fwd(tr.coarse, tr._pk[tr.coarse], raw_c, rays=(o, d, v, z_c))
+            comp_c = ops.composite(raw_c.view(1500, S, 4), z_c, d, white_bkgd=tr.white_bkgd)
             zs, z_f = ops.resample_merge(z_c, comp_c[3], Ni, det=True, seed=1)
             raw_f = torch.empty(1500 * (S + Ni), 4, device=cuda)
-            tr._fwd(tr.fine, (o, d, v, z_f), 1500 * (S + Ni), raw_f, None)
-            rgb, disp, acc, _, depth = tr._composite(raw_f, z_f, d, 1500, S + Ni)
+            launch_fwd(tr.fine, tr._pk[tr.fine], raw_f, rays=(o, d, v, z_f))
+            rgb, disp, acc, _, depth = ops.composite(raw_f.view(1500, S + Ni, 4), z_f, d, white_bkgd=tr.white_bkgd)
             torch.cuda.synchronize()
             assert torch.equal(got["rgb_map"], rgb) and torch.equal(got["acc_map"], acc)
             assert torch.equal(got["depth_map"], depth) and torch.equal(got["rgb0"], comp_c[0])

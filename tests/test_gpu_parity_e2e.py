@@ -269,6 +269,7 @@ def test_render_rays_driver_equals_the_kernel_sequence(cuda):
     host would issue one by one: every intermediate and every map must be bit-identical to that sequence -- for the
     deterministic render and for the jittered one (same Philox seeds)."""
     from ctxnerf import ops
+    from ctxnerf.mlp import launch_fwd
     from ctxnerf.train import NerfTrainer
     from ctxnerf.workloads import orbit_camera
     K, c2w = orbit_camera()
@@ -282,12 +283,12 @@ def test_render_rays_driver_equals_the_kernel_sequence(cuda):
         o, d, v, z_c = r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]
         R = o.shape[0]
         raw_c = torch.empty(R * S, 4, device=cuda)
-        tr._fwd(tr.coarse, (o, d, v, z_c), R * S, raw_c, None)
-        comp_c = tr._composite(raw_c, z_c, d, R, S)
+        launch_fwd(tr.coarse, tr._pk[tr.coarse], raw_c, rays=(o, d, v, z_c))
+        comp_c = ops.composite(raw_c.view(R, S, 4), z_c, d, white_bkgd=tr.white_bkgd)
         zs, z_f = ops.resample_merge(z_c, comp_c[3], Ni, det=not perturb, seed=seed + 1)
         raw_f = torch.empty(R * (S + Ni), 4, device=cuda)
-        tr._fwd(tr.fine, (o, d, v, z_f), R * (S + Ni), raw_f, None)
-        comp_f = tr._composite(raw_f, z_f, d, R, S + Ni)
+        launch_fwd(tr.fine, tr._pk[tr.fine], raw_f, rays=(o, d, v, z_f))
+        comp_f = ops.composite(raw_f.view(R, S + Ni, 4), z_f, d, white_bkgd=tr.white_bkgd)
         torch.cuda.synchronize()
         assert torch.equal(got["z_f"], z_f) and torch.equal(got["raw_f"], raw_f)
         for a, b in zip(got["comp_c"] + got["comp_f"], comp_c + comp_f):
@@ -302,8 +303,8 @@ def test_render_rays_driver_equals_the_kernel_sequence(cuda):
     r = ops.raygen(1024, 1024, Kv, torch.as_tensor(cv, dtype=torch.float32).to(cuda), n_samples=192, near=tr.near,
                    far=tr.far, sphere=sph, want_viewdirs=True, ray_idx=idx4)
     raw = torch.empty(3000 * 192, 4, device=cuda)
-    tr._fwd(tr.fine, (r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]), 3000 * 192, raw, None)
-    rgb, disp, acc, _, depth = tr._composite(raw, r["z_vals"], r["rays_d"], 3000, 192)
+    launch_fwd(tr.fine, tr._pk[tr.fine], raw, rays=(r["rays_o"], r["rays_d"], r["viewdirs"], r["z_vals"]))
+    rgb, disp, acc, _, depth = ops.composite(raw.view(3000, 192, 4), r["z_vals"], r["rays_d"], white_bkgd=tr.white_bkgd)
     torch.cuda.synchronize()
     assert torch.equal(got["rgb_map"], rgb) and torch.equal(got["acc_map"], acc) and torch.equal(got["depth_map"], depth)
     assert torch.equal(torch.nan_to_num(got["disp_map"]), torch.nan_to_num(disp))
