@@ -75,6 +75,14 @@ _SIGNATURES = {
     "ctx_render_args_bytes": (c_int, []),
     "ctx_image_metrics": (c_int, [P, P, c_int, c_int, c_int, c_int, P, P, P, P]),
     "ctx_image_metrics_partials": (c_int64, [c_int, c_int, c_int]),
+    "ctx_density_grid_workspace": (c_int64, [c_int, c_int, c_int]),
+    "ctx_density_grid": (c_int, [P, c_int, c_int, c_int, c_int, c_int, c_float, c_float, c_float, c_float, c_float,
+                                 c_float, P, c_int64, P, P]),
+    "ctx_marching_cubes_workspace": (c_int64, [c_int, c_int, c_int]),
+    "ctx_marching_cubes": (c_int, [P, c_int, c_int, c_int, c_float, c_float, c_float, c_float, c_float, c_float,
+                                   c_float, P, c_int64, P, P, P, P, c_int, P]),
+    "ctx_vertex_colors_workspace": (c_int64, [c_int64]),
+    "ctx_vertex_colors": (c_int, [P, c_int, c_int, P, P, c_int64, P, c_int64, P, P]),
     "ctx_comm_load": (c_int, [ctypes.c_char_p]),
     "ctx_comm_version": (c_int, []),
     "ctx_comm_last_error": (ctypes.c_char_p, []),

@@ -23,7 +23,7 @@ from typing import Optional
 
 import torch
 
-from . import _lib, ops
+from . import _lib, mesh, ops
 from ._lib import CtxNerfError, call, ptr, stream_ptr
 from .dist import BucketComm, FlatBucket, dist_backend, world
 from .mlp import launch_fwd, pack_into
@@ -598,3 +598,40 @@ class NerfTrainer:
             return dict(rgb_map=rgb.reshape(H, W, 3), disp_map=disp.reshape(H, W), acc_map=acc.reshape(H, W),
                         depth_map=depth.reshape(H, W))
         return dict(rgb_map=rgb, disp_map=disp, acc_map=acc, depth_map=depth)
+
+    # ------------------------------------------------------------ geometry
+    def _mesh_net(self, network, what):
+        if self.ndc:
+            raise CtxNerfError(f"NerfTrainer.{what}: an ndc=True trainer's field lives in NDC space, so a lattice over "
+                               "world bounds would not sample it")
+        nets = {"fine": self.fine, "coarse": self.coarse}
+        if network not in nets:
+            raise CtxNerfError(f"NerfTrainer.{what}: network must be 'fine' or 'coarse', got {network!r}")
+        return nets[network]
+
+    @torch.no_grad()
+    def density_grid(self, resolution=256, bounds=mesh.DEFAULT_BOUNDS, network="fine"):
+        """``relu(sigma)`` of the ``network`` ('fine' or 'coarse') on a lattice of ``resolution`` cells (an int or
+        ``(nx, ny, nz)``) over ``bounds = (lo, hi)``, with zero view directions, as the original NeRF release's
+        ``extract_mesh.ipynb``: fp32 ``[nx+1, ny+1, nz+1]`` on the device (``ctxnerf.mesh.density_grid`` on the
+        trainer's packed weights).  The training state is left as it was, and no collective is entered."""
+        net = self._mesh_net(network, "density_grid")
+        with torch.cuda.device(self.device):
+            return mesh.density_grid(net, self._pk[net], resolution, bounds)
+
+    @torch.no_grad()
+    def extract_mesh(self, resolution=256, bounds=mesh.DEFAULT_BOUNDS, threshold=50.0, network="fine", colors=True):
+        """The surface ``sigma == threshold`` of ``density_grid(resolution, bounds, network)`` by marching cubes
+        (upstream thresholds the relu'd density at 50), with a colour per vertex: ``sigmoid(rgb)`` of the same network
+        seen along ``-normal``.  Returns ``dict(vertices [V,3], faces [F,3] int32, normals [V,3], colors [V,3] or
+        None)`` on the device; ``ctxnerf.mesh.write_ply`` writes it.  The training state is left as it was."""
+        net = self._mesh_net(network, "extract_mesh")
+        if not float(threshold) > 0.0:
+            raise CtxNerfError(f"NerfTrainer.extract_mesh: threshold must be > 0 (the density is relu'd), got "
+                               f"{threshold}")
+        mesh.lattice(bounds, mesh._cells(resolution))      # refuse bad bounds before any launch
+        with torch.cuda.device(self.device):
+            sigma = mesh.density_grid(net, self._pk[net], resolution, bounds)
+            out = mesh.marching_cubes(sigma, threshold, bounds)
+            out["colors"] = mesh.vertex_colors(net, self._pk[net], out["vertices"], out["normals"]) if colors else None
+        return out

@@ -351,6 +351,48 @@ int ctx_image_metrics(const float* pred, const void* target, int target_u8, int 
                       double* mse, double* ssim, double* partials, void* stream);
 int64_t ctx_image_metrics_partials(int B, int H, int W);   /* -1 for B < 0, H < 1 or W < 1 */
 
+/* ---- mesh extraction: the original NeRF release's extract_mesh.ipynb (density of the fine network on a regular
+ * lattice with zero view directions, relu, PyMCubes marching_cubes(sigma, threshold), index -> world coordinates) and
+ * a colour per vertex.  Lattice: (nx+1) x (ny+1) x (nz+1) points in C order, point (i, j, k) at
+ * (ox + hx*i, oy + hy*j, oz + hz*k) formed in fp32 as __fadd_rn(o, __fmul_rn(h, (float)i)).
+ *
+ * ctx_density_grid: sigma [nx+1, ny+1, nz+1] fp32 = relu(raw[..., 3]) of `net` (a 4-channel net; L_pts / L_dirs its
+ * encoding frequencies).  Lattice column (i, j) runs through ctx_mlp_fwd_ex mode 1 as the ray o = (x_i, y_j, 0),
+ * d = (0, 0, 1) with the depth row z_k and a zero view direction; the view head is computed and discarded.  The work
+ * goes in slabs of x-planes through the caller's workspace (256-byte aligned) of at least
+ * ctx_density_grid_workspace(nx, ny, nz) bytes (one plane); a larger one takes bigger slabs.  The result is the same
+ * bit for bit whatever the workspace size.  Bad arguments (before any launch): a cell count per axis outside
+ * [1, 1024], a lattice of 2^31 points or more, a null / unsuitable net, a short or misaligned workspace.           */
+int64_t ctx_density_grid_workspace(int nx, int ny, int nz);   /* -1 for sizes outside the limits above */
+int ctx_density_grid(const CtxNet* net, int L_pts, int L_dirs, int nx, int ny, int nz, float ox, float oy, float oz,
+                     float hx, float hy, float hz, void* workspace, int64_t workspace_bytes, float* sigma,
+                     void* stream);
+/* ctx_marching_cubes: the iso-surface sigma == iso of the lattice sigma [nx+1, ny+1, nz+1] (nx, ny, nz >= 1, fewer than
+ * 2^31 points) placed as above.  Case table and rule: csrc/mc_tables.cuh (generated by oracle/mc_tables.py; corner c
+ * at offset (c & 1, c >> 1 & 1, c >> 2 & 1), inside iff sigma >= iso, ambiguous faces separate the inside corners, so
+ * neighbouring cells agree and the mesh has no cracks; triangle normals point towards decreasing density).
+ * pass 0 counts: counts[0] = V (vertices), counts[1] = F (triangles), int64 on the device; read them back and allocate.
+ * pass 1 writes vertices [V,3] fp32 (world coordinates), normals [V,3] fp32 (nullable) and faces [F,3] int32 (the
+ *   caller checks V < 2^31).
+ * Order: one vertex per lattice edge whose ends straddle iso, numbered by (linear index of the lower endpoint, then
+ * axis x < y < z); position t = (iso - s0) / (s1 - s0) (IEEE division), then o + h * (idx + t) with one rounding per
+ * operation.  The normal is the normalised negative density gradient (central differences, one-sided on the lattice
+ * border, divided by the spacing), linearly interpolated along the edge; a zero gradient gives (0, 0, 0).  Faces come
+ * in cell order, then in table order.  oracle/marching_cubes.py restates all of it bit for bit.
+ * workspace: caller-owned, 256-byte aligned, ctx_marching_cubes_workspace(nx, ny, nz) bytes (about 2.5 bytes per
+ * lattice point), the same buffer for both passes.  No atomics: the output is the same on every run.             */
+int64_t ctx_marching_cubes_workspace(int nx, int ny, int nz);   /* -1 for sizes outside the limits above */
+int ctx_marching_cubes(const float* sigma, int nx, int ny, int nz, float ox, float oy, float oz, float hx, float hy,
+                       float hz, float iso, void* workspace, int64_t workspace_bytes, int64_t* counts, float* vertices,
+                       float* normals, int* faces, int pass, void* stream);
+/* ctx_vertex_colors: rgb [V,3] = sigmoid(raw[:, :3]) of `net` at each vertex [V,3] seen along -normal (normals
+ * nullable: a zero view direction), through ctx_mlp_fwd_ex mode 1 with S = 1, o = vertex, d = 0, z = 0.  Chunks of
+ * vertices go through the caller's workspace (256-byte aligned, at least ctx_vertex_colors_workspace(1) bytes;
+ * ctx_vertex_colors_workspace(n) holds a chunk of n); the result is the same whatever its size.                    */
+int64_t ctx_vertex_colors_workspace(int64_t n_vertices);   /* -1 for n_vertices < 1 */
+int ctx_vertex_colors(const CtxNet* net, int L_pts, int L_dirs, const float* vertices, const float* normals,
+                      int64_t V, void* workspace, int64_t workspace_bytes, float* rgb, void* stream);
+
 /* ---- gradient all-reduce (SURVEY.md 8b / 8e): the one exchange step of the ray-sharded training step, replacing the
  * reduce-add of nn.DataParallel (src/training/trainer.py:134-135).  NCCL is opened at run time (dlopen; `path`
  * nullable = "libnccl.so.2" by soname), so the library has no link-time dependency on it; every call below returns
